@@ -2,7 +2,7 @@
 """Headline benchmark of the Marlin-prover hot path on B200: BLS12-377 G1 variable-base MSM, with the
 NTT and the whole Marlin prover (setup / index / prove / verify) measured beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n 26] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--log-n 26] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -27,6 +27,10 @@ single-GPU size.  Scalars are uniform in [0, r).
   extra.marlin the prover end to end at 2^20 constraints on the GPU and on the CPU arm (same proof
                bytes), and the reference's own bound universal_setup(100000, 25000, 300000) with
                setup + index + prove + verify timed as one unit (what its tests pay per call)
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the MSM result of the last timed step to DIR/msm_result.npy
+(see dump_outputs).  Bases and scalars come from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 
 --impl reference: the CPU arm alone (arkworks-equivalent C port on all host cores; under torchrun
 rank 0 runs it, the other ranks exit) on the same config and metric.
@@ -163,6 +167,18 @@ def workload_config(log_n: int) -> dict:
             "bases": "SRS powers beta^i*G",
             "l2": "a 256 MiB buffer is rewritten between timed steps and the inputs (2 GiB of scalars, 66 GiB of table "
                   "records at 2^26) exceed the 126 MB L2 anyway"}
+
+
+def dump_outputs(out_dir: str, result: np.ndarray) -> None:
+    """DIR/msm_result.npy: float64 of shape (2, 24), the affine x and y of the (1, 18) Jacobian point the MSM returned,
+    in canonical (not Montgomery) form, each as 24 little-endian 16-bit limbs, so every value is exact.  The Jacobian
+    coordinates of a point are not unique, its affine ones are.  The point at infinity is written as (0, 0), which is
+    not on the curve."""
+    from oracle import pyoracle as O
+    point = O.points_from_jacobian(result)[0] or (0, 0)
+    limbs = np.array([[(c >> (16 * j)) & 0xFFFF for j in range(24)] for c in point], dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "msm_result.npy"), limbs)
 
 
 def marlin_gpu_run(be, lg, proofs):
@@ -381,8 +397,14 @@ def main():
                          "buckets; 'index' = contiguous index ranges (round-1 behaviour; the fallback without tables)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the MSM result of the last timed step to DIR/msm_result.npy (float64, see dump_outputs)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's result; --impl reference sizes its sample by time")
     if os.environ.get("SWB_BENCH_FAULT_S"):     # debugging aid: dump every thread's Python stack if the run stalls
         import faulthandler
         faulthandler.dump_traceback_later(int(os.environ["SWB_BENCH_FAULT_S"]), exit=True)
@@ -632,6 +654,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, result)
 
     # ---- roofline of the dominant kernel -------------------------------------------------------------
     # limb-products/s the integer pipe can issue: IMAD.WIDE.U32 (one 32x32+64 per instruction),

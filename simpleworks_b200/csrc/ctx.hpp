@@ -58,8 +58,7 @@ struct swb_ctx {
         bool active = false, empty = false;
     } msm_slot[MSM_SLOTS];
     int scratch_slot = 0;              // suffix of scratch tags while a slot > 0 is being launched
-    // bucket sharding (swb_msm_set_bucket_shard): MSMs on this context only fill the buckets b with
-    // b mod world == rank of every bucket set and return that share of the result
+    // bucket sharding of the swb_msm_* entry points (swb_msm_set_bucket_shard, swb::BucketShard)
     int bucket_rank = 0, bucket_world = 1;
     // multi-GPU proving (swb_set_msm_shard): this rank's share of every prover MSM, and who adds them up
     int shard_rank = 0, shard_world = 1;
@@ -93,17 +92,24 @@ int set_err(swb_ctx* c, int code, const char* fmt, ...);
 // wait for the context's stream and for the MSM slots' own streams (before device memory they may be
 // reading is released)
 void sync_all_streams(swb_ctx* c);
+// A bucket shard: the MSM fills only the buckets b with b mod world == rank of every bucket set and returns that share of
+// the result (world a power of two; world = 1: all buckets)
+struct BucketShard { int rank, world; };
 // One MSM split in two: msm_begin enqueues everything up to the device->host copy of the bucket-set
 // sums (slot 0: on the context's stream; slot > 0: on the slot's own streams, after the work already
 // queued on the context's stream), msm_end waits for it and finishes on the host.  A slot holds one
 // MSM at a time.
-int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery);
+int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
+              BucketShard shard);
 // Several scalar vectors over one handle WITH window tables as ONE MSM pipeline (one sort, one accumulation, one bucket
 // reduction; a bucket set per vector): msm_end then delivers `count` results.  msm_can_batch says whether a list qualifies.
 bool msm_can_batch(swb_ctx* c, const swb_bases* bases, size_t count, const size_t* ns);
 int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, const size_t* offsets, const void* const* scalars_dev,
-                    const size_t* ns, int montgomery);
+                    const size_t* ns, int montgomery, BucketShard shard);
 int msm_end(swb_ctx* c, int slot, swb_g1_jacobian* out);
+// fixed_base.cu: the window-table width that suits MSMs of about n scalars (what swb_bases_precompute picks for
+// window_bits = 0)
+int tables_pick_window(size_t n);
 // Device blocks for short-lived vectors (the prover allocates and frees hundreds per proof).  All work of
 // a context is ordered on one stream, so a freed block can be handed to the next request at once;
 // blocks are rounded to 2 MiB and kept until swb_destroy, which keeps cudaMalloc/cudaFree (and the

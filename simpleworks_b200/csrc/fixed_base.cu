@@ -127,6 +127,7 @@ __global__ void k_bases_export(uint8_t* __restrict__ out, const Fq* __restrict__
 // per base: c doublings per level in XYZZ, then one inversion for the base's W - 1 new points
 // (Montgomery's trick over zz*zzz).
 constexpr int TAB_MAX_LEVELS = 32;
+static_assert((253 + 8 - 1) / 8 <= TAB_MAX_LEVELS, "swb_bases_precompute accepts window widths from 8 bits on");
 __global__ void __launch_bounds__(128) k_bases_tables(Fq* __restrict__ tab, size_t N, int c, int W) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
@@ -286,9 +287,9 @@ extern "C" int swb_bases_export(swb_ctx* c, const swb_bases* b, size_t offset, s
     return SWB_OK;
 }
 
-// pick the digit width that minimises (additions) + (bucket work) for MSMs over all N bases; the
+// the digit width that minimises (additions) + (bucket work) for MSMs of N scalars over window tables; the
 // two weights are the measured cost of one mixed addition and of one bucket in gather + reduce
-static int tables_pick_window(size_t N) {
+int swb::tables_pick_window(size_t N) {
     int best = 8;
     double best_cost = 1e300;
     for (int cb = 8; cb <= 23; cb++) {
@@ -303,12 +304,11 @@ extern "C" int swb_bases_precompute(swb_ctx* c, swb_bases* b, int window_bits) {
     if (!c) return SWB_EARG;
     SWB_REQUIRE(c, b != nullptr, "bases_precompute: NULL bases");
     SWB_REQUIRE(c, b->ctx == c, "bases_precompute: bases belong to another context");
-    SWB_REQUIRE(c, window_bits == 0 || (window_bits >= 4 && window_bits <= 24), "bases_precompute: window_bits must be 0 or in [4,24]");
+    SWB_REQUIRE(c, window_bits == 0 || (window_bits >= 8 && window_bits <= 24), "bases_precompute: window_bits must be 0 or in [8,24]");
     if (b->tab_w) return SWB_OK;                 // already built
     if (b->n == 0) return SWB_OK;
     const int cb = window_bits ? window_bits : tables_pick_window(b->n);
     const int W = (253 + cb - 1) / cb;
-    SWB_REQUIRE(c, W <= TAB_MAX_LEVELS, "bases_precompute: too many levels for this window width");
     SWB_REQUIRE(c, b->n * (size_t)W < ((size_t)1 << 31), "bases_precompute: n * levels must be < 2^31");
     SWB_CUDA(c, cudaSetDevice(c->device));
     Fq* tab = nullptr;

@@ -23,7 +23,8 @@
 //     void  bases_tune(void* h, size_t typical_n);   // optional restructuring for MSMs of about typical_n scalars
 //     size_t msm_submit(void* h, size_t offset, const Vec& scalars, size_t n);   // queue an MSM (scalars stay alive)
 //     G1Point msm_result(size_t id);  void msm_drain();
-//     G1Point msm(void* h, size_t offset, const Vec& scalars_mont, size_t n);  // sum s_i * base[offset+i]
+//     // sum s_i * base[offset+i]; needed only by engines whose msm_submit is msm_submit_sync (vec_host.hpp)
+//     G1Point msm(void* h, size_t offset, const Vec& scalars_mont, size_t n);
 //   };
 //
 // Verification is the pairing check of kzg10::batch_check on the host (marlin/pairing.hpp): the two

@@ -394,19 +394,13 @@ struct GpuEngine {
     }
     void free_bases(void* h) { swb_bases_free(static_cast<swb_bases*>(h)); }
     // window tables (swb_bases_precompute) with the digit width that suits MSMs of about typical_n
-    // scalars: same cost model as the library's own choice (0.37 ns per addition, 3.7 ns per bucket).
-    // KZG powers lie in the prime-order subgroup (g is cofactor-cleared), which the tables require.
+    // scalars (tables_pick_window).  KZG powers lie in the prime-order subgroup (g is cofactor-cleared), which the
+    // tables require.
     // Skipped silently when they would not fit in half of the free device memory.
     void bases_tune(void* h, size_t typical_n) {
         swb_bases* b = static_cast<swb_bases*>(h);
         if (!b || typical_n == 0) return;
-        int best = 0;
-        double best_cost = 1e300;
-        for (int cb = 8; cb <= 23; cb++) {
-            const int W = (253 + cb - 1) / cb;
-            const double cost = (double)typical_n * W * 0.37 + (double)((size_t)1 << (cb - 1)) * 3.7;
-            if (cost < best_cost) { best_cost = cost; best = cb; }
-        }
+        const int best = tables_pick_window(typical_n);
         const size_t W = (253 + best - 1) / best;
         size_t free_b = 0, total_b = 0;
         cudaSetDevice(c->device);
@@ -450,13 +444,16 @@ struct GpuEngine {
         return p;
     }
     bool sharding() const { return c->shard_world > 1 && (c->shard_combine || c->comm); }
-    // Power-of-two worlds shard by BUCKET (swb_msm_set_bucket_shard: every rank sees the whole polynomial -- it
+    // Power-of-two worlds shard by BUCKET (swb::BucketShard: every rank sees the whole polynomial -- it
     // has it anyway -- and fills its interleaved share of the buckets, so accumulation AND bucket reduction shrink
     // and the window width stays that of one GPU); other worlds by contiguous index range.
+    bool shards_by_bucket() const { return sharding() && (c->shard_world & (c->shard_world - 1)) == 0; }
     // (only over bases with window tables: on the plain path every rank would still sort all pairs, and the index
     // split measured slightly faster -- 2^20 constraints on two GPUs: 0.248 s against 0.256 s)
-    bool bucket_mode(const swb_bases* b) const {
-        return sharding() && b && b->tab_w > 0 && (c->shard_world & (c->shard_world - 1)) == 0 && !getenv("SWB_SHARD_INDEX");
+    bool bucket_mode(const swb_bases* b) const { return shards_by_bucket() && b && b->tab_w > 0; }
+    // the bucket shard ticket t runs under: this rank's share for a by-bucket ticket, else the context's own
+    BucketShard bucket_shard(const Ticket& t) const {
+        return t.by_bucket ? BucketShard{c->shard_rank, c->shard_world} : BucketShard{c->bucket_rank, c->bucket_world};
     }
     void finish(Ticket& t) {
         t.done = true;
@@ -482,10 +479,7 @@ struct GpuEngine {
         size_t off, n;
         const Fr* sc;
         local_part(t, &off, &sc, &n);
-        if (t.by_bucket) { c->bucket_rank = c->shard_rank; c->bucket_world = c->shard_world; }
-        const int rc = msm_begin(c, slot, static_cast<swb_bases*>(t.h), off, sc, n, 1);
-        if (t.by_bucket) { c->bucket_rank = 0; c->bucket_world = 1; }     // the plan of this MSM has captured it
-        ck(rc, "msm");
+        ck(msm_begin(c, slot, static_cast<swb_bases*>(t.h), off, sc, n, 1, bucket_shard(t)), "msm");
         t.launched = true;
         t.slot = slot;
         slot_owner[slot] = (long)id;
@@ -511,10 +505,7 @@ struct GpuEngine {
                 // the slots must be idle: the batch runs on the context's stream with slot 0's scratch
                 for (int sl = 1; sl < swb_ctx::MSM_SLOTS; sl++)
                     if (slot_owner[sl] >= 0) collect((size_t)slot_owner[sl]);
-                if (tickets[k].by_bucket) { c->bucket_rank = c->shard_rank; c->bucket_world = c->shard_world; }
-                int rc = msm_begin_batch(c, 0, b, e - k, offs.data(), scs.data(), ns.data(), 1);
-                if (tickets[k].by_bucket) { c->bucket_rank = 0; c->bucket_world = 1; }
-                ck(rc, "msm (batch)");
+                ck(msm_begin_batch(c, 0, b, e - k, offs.data(), scs.data(), ns.data(), 1, bucket_shard(tickets[k])), "msm (batch)");
                 std::vector<swb_g1_jacobian> outs(e - k);
                 ck(msm_end(c, 0, outs.data()), "msm (batch)");
                 for (size_t q = k; q < e; q++) {
@@ -569,7 +560,7 @@ struct GpuEngine {
     }
     // (sizes the SRS window tables: in a power-of-two world they will be used by bucket, i.e. on whole polynomials)
     size_t msm_local_count(size_t n) {
-        if (!sharding() || ((c->shard_world & (c->shard_world - 1)) == 0 && !getenv("SWB_SHARD_INDEX"))) return n;
+        if (!sharding() || shards_by_bucket()) return n;
         const size_t base = n / (size_t)c->shard_world, rem = n % (size_t)c->shard_world;
         return base + ((size_t)c->shard_rank < rem ? 1 : 0);
     }
@@ -602,20 +593,6 @@ struct GpuEngine {
     }
     ~GpuEngine() {
         try { msm_drain(); } catch (...) {}
-    }
-    G1Point msm(void* h, size_t offset, const Vec& scalars, size_t n) {
-        OpTimer ot_(c, "msm");
-        swb_g1_jacobian out;
-        ck(swb_msm_g1_fr_dev(c, static_cast<swb_bases*>(h), offset, reinterpret_cast<const swb_fr*>(scalars.p), n, &out), "msm");
-        G1Point p = G1Point::identity();
-        Fq z;
-        memcpy(z.l, out.z.l, 48);
-        if (!z.is_zero()) {                 // the library returns Z = 1
-            p.infinity = false;
-            memcpy(p.x.l, out.x.l, 48);
-            memcpy(p.y.l, out.y.l, 48);
-        }
-        return p;
     }
 };
 using Api = MarlinApi<GpuEngine>;

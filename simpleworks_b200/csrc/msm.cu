@@ -6,7 +6,8 @@
 // c-bit windows with 2^c - 1 Jacobian buckets per window and one rayon task per window; here:
 //
 //   1. k_msm_digits        scalars -> signed c-bit digits (halves the bucket count); one
-//                           (bucket, point index | sign) pair per scalar and window, window-major
+//                           (bucket, point index | sign) pair per scalar and window, window-major; one
+//                           instance per width c, which is a template parameter
 //   2. radix_sort_segmented pairs grouped by bucket inside each window (radix_sort.cu)
 //   3. k_msm_range_count    the sorted positions are cut into fixed-length ranges; runs per range,
 //                           exclusive scan = where each range writes its partial sums
@@ -84,30 +85,82 @@ static int slot_prepare(swb_ctx* c, int slot) {
     return SWB_OK;
 }
 
-// smallest number of sorted pairs from which pair sums run automatically (SWB_PAIR_MIN_LOG: tuning aid)
-static size_t msm_pair_min_total() {
-    static const size_t v = [] {
-        const char* e = getenv("SWB_PAIR_MIN_LOG");
-        const long l = e ? atol(e) : 24;
-        return (size_t)1 << (l >= 10 && l <= 40 ? l : 24);
-    }();
-    return v;
-}
+static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBatch& batch, BucketShard shard, int montgomery);
 
-static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBatch& batch, int montgomery);
+// The table rule: window tables pay once the buckets hold a few points each (n * W >= 8 * 2^(c-1) per bucket set), unless
+// swb_msm_set_table_policy or a window width set with swb_msm_set_window_bits says otherwise.
+static bool msm_use_tables(const swb_ctx* c, const swb_bases* b, size_t n, size_t sets) {
+    return b->tab_w > 0 && !c->msm_window_override && c->msm_table_policy >= 0 &&
+           (c->msm_table_policy > 0 || n * (size_t)b->tab_w >= ((size_t)8 << (b->tab_c - 1)) * sets);
+}
 
 // can these vectors run as ONE batched MSM (one bucket set each over the handle's window tables)?
 bool msm_can_batch(swb_ctx* c, const swb_bases* bases, size_t count, const size_t* ns) {
-    if (!bases || bases->tab_w == 0 || c->msm_window_override || c->msm_table_policy < 0 || count < 2 || count > (size_t)MSM_MAX_BATCH) return false;
+    if (!bases || count < 2 || count > (size_t)MSM_MAX_BATCH) return false;
     size_t total = 0;
     for (size_t k = 0; k < count; k++) total += ns[k];
-    // the shared rule of the table path, for the batch as a whole: a few points per bucket
-    return total < ((size_t)1 << 31) &&
-           (c->msm_table_policy > 0 || total * (size_t)bases->tab_w >= ((size_t)8 << (bases->tab_c - 1)) * count);
+    return total < ((size_t)1 << 31) && msm_use_tables(c, bases, total, count);
+}
+
+void msm_plan_pairs(const swb_ctx* c, MsmPlan& pl) {
+    // enough threads to fill the GPU (>= ~512 per SM) but at most 128 additions each
+    const size_t want = pl.total / ((size_t)c->sm_count * 512);
+    uint32_t len = 16;
+    while (len < 128 && len < want) len <<= 1;
+    pl.range_len = len;
+    pl.nranges = (uint32_t)((pl.total + len - 1) / len);
+    // batch-affine pair sums first when buckets are well filled and the input is large enough to amortise the block-wide
+    // inversions (swb_msm_set_pair_sums: 0 never, 1 automatic, 1 + k forces k levels)
+    int levels = 0;
+    if (c->msm_pair_policy >= 2) levels = c->msm_pair_policy - 1;
+    else if (c->msm_pair_policy == 1 && pl.total >= MSM_PAIR_MIN_PAIRS) {
+        // a level pays while most aligned blocks of 2^L positions still lie inside one bucket
+        const double per_bucket = pl.nb ? (double)pl.total / (double)pl.nb : 0.0;
+        while (levels < MSM_PAIR_MAX_LEVELS && per_bucket >= (double)(8u << levels)) levels++;
+    }
+    pl.pair_levels = pl.total >= 2 ? levels : 0;
+}
+
+// Every decision of one MSM, from the context's settings, the bases, the batch and the bucket shard.  Under compaction
+// the number of pairs is known only after the digits kernel: the sizes planned here are then upper bounds for the
+// scratch, and msm_launch_digits_sort plans the ranges and pair sums again.
+static int msm_plan(swb_ctx* c, const swb_bases* bases, const MsmBatch& batch, BucketShard shard, MsmPlan& pl) {
+    pl = MsmPlan{};
+    pl.n = batch.start[batch.count];
+    const bool tables = batch.count > 1 || msm_use_tables(c, bases, pl.n, 1);    // a batch always runs over tables
+    pl.cb = tables ? bases->tab_c : pick_window(c, pl.n);
+    pl.ndig = tables ? bases->tab_w : (254 + pl.cb - 1) / pl.cb;
+    pl.nwin = tables ? (int)batch.count : pl.ndig;        // bucket sets
+    SWB_REQUIRE(c, pl.ndig <= MSM_MAX_WINDOWS, "msm: too many windows");
+    pl.tab_stride = tables ? bases->n : 0;
+    pl.B = 1u << (pl.cb - 1);
+    if (shard.world > 1 && (uint32_t)shard.world <= pl.B / 2) {
+        // bucket sharding: this rank fills the buckets b = rank (mod world) of every set.  On the table path (one
+        // set, pair order free) the other ranks' pairs are dropped right in the digits kernel.
+        while ((1 << pl.shard_shift) < shard.world) pl.shard_shift++;
+        pl.B >>= pl.shard_shift;
+        pl.shard_rank = (uint32_t)shard.rank;
+        pl.compact = tables;
+    } else if (shard.world > 1 && shard.rank != 0) {
+        pl.idle = true;           // too few buckets to split (tiny MSM, narrow window)
+        return SWB_OK;
+    }
+    pl.nb = (uint32_t)pl.nwin * pl.B;
+    pl.key_space = tables ? pl.nb : pl.B;     // table path: one segment, the key says which set; plain path: a segment per set
+    pl.total = pl.n * (size_t)pl.ndig;
+    pl.seg_len = tables ? pl.total : pl.n;
+    SWB_REQUIRE(c, pl.total < ((size_t)1 << 32), "msm: n * windows must be < 2^32");
+    msm_plan_pairs(c, pl);
+    if (pl.compact) {       // whatever number of pairs survives: at most this many ranges
+        const size_t a = pl.total / 128 + 1, b = (size_t)c->sm_count * 512 + 1;
+        pl.nranges = (uint32_t)(a > b ? a : b);
+    }
+    pl.pcap = pl.nranges + pl.nb;
+    return SWB_OK;
 }
 
 int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, const size_t* offsets, const void* const* scalars_dev,
-                    const size_t* ns, int montgomery) {
+                    const size_t* ns, int montgomery, BucketShard shard) {
     SWB_REQUIRE(c, slot >= 0 && slot < swb_ctx::MSM_SLOTS, "msm: bad slot");
     SWB_REQUIRE(c, !c->msm_slot[slot].active, "msm: slot already holds an MSM");
     SWB_REQUIRE(c, bases != nullptr && count >= 1 && count <= (size_t)MSM_MAX_BATCH && offsets && scalars_dev && ns, "msm: bad batch");
@@ -148,15 +201,16 @@ int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, 
         c->stream = sl.work;
         c->scratch_slot = slot;
     }
-    rc = msm_enqueue(c, slot, bases, batch, montgomery);
+    rc = msm_enqueue(c, slot, bases, batch, shard, montgomery);
     c->stream = main_stream;
     c->scratch_slot = 0;
     if (rc == SWB_OK) sl.active = true;
     return rc;
 }
 
-int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery) {
-    return msm_begin_batch(c, slot, bases, 1, &offset, &scalars_dev, &n, montgomery);
+int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
+              BucketShard shard) {
+    return msm_begin_batch(c, slot, bases, 1, &offset, &scalars_dev, &n, montgomery, shard);
 }
 
 // outs: one result per vector of the batch (one for a plain msm_begin)
@@ -207,65 +261,39 @@ int msm_end(swb_ctx* c, int slot, swb_g1_jacobian* out) {
     return SWB_OK;
 }
 
+// the bucket shard of swb_msm_set_bucket_shard, under which the swb_msm_* entry points run
+static BucketShard ctx_bucket_shard(const swb_ctx* c) { return {c->bucket_rank, c->bucket_world}; }
+
 static int msm_run(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
                    swb_g1_jacobian* out) {
     SWB_REQUIRE(c, out != nullptr, "msm: NULL argument");
-    int rc = msm_begin(c, 0, bases, offset, scalars_dev, n, montgomery);
+    int rc = msm_begin(c, 0, bases, offset, scalars_dev, n, montgomery, ctx_bucket_shard(c));
     if (rc != SWB_OK) return rc;
     return msm_end(c, 0, out);
 }
 
-static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBatch& batch, int montgomery) {
+// scalars in host memory (32 bytes each): copied to device scratch first
+static int msm_run_host(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_host, size_t n, int montgomery,
+                        swb_g1_jacobian* out) {
+    SWB_REQUIRE(c, n == 0 || scalars_host != nullptr, "msm: NULL scalars");
+    void* d = nullptr;
+    if (n) {
+        SWB_CUDA(c, cudaSetDevice(c->device));
+        d = get_scratch(c, "msm_scalars", n * 32);
+        if (!d) return SWB_ENOMEM;
+        SWB_CUDA(c, cudaMemcpyAsync(d, scalars_host, n * 32, cudaMemcpyHostToDevice, c->stream));
+    }
+    return msm_run(c, bases, offset, d, n, montgomery, out);
+}
+
+static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBatch& batch, BucketShard shard, int montgomery) {
     swb_ctx::MsmSlot& sl = c->msm_slot[slot];
-    const size_t n = batch.start[batch.count];
-    const bool batched = batch.count > 1;
-    // window tables are worth it once the shared buckets hold a few points each (a batch always runs over them)
-    const bool tables = batched || (bases->tab_w > 0 && !c->msm_window_override && c->msm_table_policy >= 0 &&
-                                    (c->msm_table_policy > 0 || n * (size_t)bases->tab_w >= ((size_t)8 << (bases->tab_c - 1))));
-    const int cb = tables ? bases->tab_c : pick_window(c, n);
-    const int ndig = tables ? bases->tab_w : (254 + cb - 1) / cb;
-    const int nwin = tables ? (int)batch.count : ndig;        // bucket sets
-    SWB_REQUIRE(c, ndig <= MSM_MAX_WINDOWS, "msm: too many windows");
-    MsmPlan pl{};
-    pl.n = n;
-    pl.cb = cb;
-    pl.ndig = ndig;
-    pl.nwin = nwin;
-    pl.tab_stride = tables ? bases->n : 0;
-    pl.B = 1u << (cb - 1);
-    pl.shard_rank = 0;
-    pl.shard_shift = 0;
-    pl.compact = false;
-    if (c->bucket_world > 1 && (uint32_t)c->bucket_world <= pl.B / 2) {
-        // bucket sharding: this rank fills the buckets b = rank (mod world) of every set.  On the table path (one
-        // set, pair order free) the other ranks' pairs are dropped right in the digits kernel.
-        while ((1 << pl.shard_shift) < c->bucket_world) pl.shard_shift++;
-        pl.B >>= pl.shard_shift;
-        pl.shard_rank = (uint32_t)c->bucket_rank;
-        pl.compact = tables;
-    } else if (c->bucket_world > 1 && c->bucket_rank != 0) {
-        // too few buckets to split (tiny MSM, narrow window): rank 0 computes all of it, the others contribute the identity
+    MsmPlan pl;
+    int rc = msm_plan(c, bases, batch, shard, pl);
+    if (rc != SWB_OK) return rc;
+    if (pl.idle) {
         sl.empty = true;
         return SWB_OK;
-    }
-    pl.nb = (uint32_t)nwin * pl.B;
-    pl.key_space = tables ? pl.nb : pl.B;     // table path: one segment, the key says which set; plain path: a segment per set
-    pl.total = n * (size_t)ndig;
-    pl.seg_len = tables ? pl.total : n;
-    SWB_REQUIRE(c, pl.total < ((size_t)1 << 32), "msm: n * windows must be < 2^32");
-    {
-        // enough threads to fill the GPU (>= ~512 per SM) but at most 128 additions each (re-planned after the digits
-        // kernel when it compacts; these are then upper bounds for the scratch sizes)
-        size_t want = pl.total / ((size_t)c->sm_count * 512);
-        uint32_t len = 16;
-        while (len < 128 && len < want) len <<= 1;
-        pl.range_len = len;
-        pl.nranges = (uint32_t)((pl.total + len - 1) / len);
-        if (pl.compact) {       // whatever number of pairs survives: at most this many ranges (see msm_plan_ranges)
-            const size_t a = pl.total / 128 + 1, b = (size_t)c->sm_count * 512 + 1;
-            pl.nranges = (uint32_t)(a > b ? a : b);
-        }
-        pl.pcap = pl.nranges + pl.nb;
     }
     MsmBuffers bf{};
     bf.keys = (uint32_t*)get_scratch(c, "msm_keys", msm_alt_offset(pl.total) * 4 * 2);
@@ -277,9 +305,9 @@ static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBa
     bf.partial = (G1Xyzz*)get_scratch(c, "msm_partial", (size_t)pl.pcap * sizeof(G1Xyzz));
     bf.buckets = (G1Xyzz*)get_scratch(c, "msm_buckets", (size_t)pl.nb * sizeof(G1Xyzz));
     {
-        const size_t segs = (size_t)nwin * (pl.B / msm_reduce_seg_len((uint32_t)nwin, pl.B));
+        const size_t segs = (size_t)pl.nwin * (pl.B / msm_reduce_seg_len((uint32_t)pl.nwin, pl.B));
         bf.seg = (G1Xyzz*)get_scratch(c, "msm_seg", (2 * segs + 2) * sizeof(G1Xyzz));
-        bf.seg2 = (G1Xyzz*)get_scratch(c, "msm_seg2", ((size_t)nwin * 24 * 33 + 2) * sizeof(G1Xyzz));   // [sets][jobs][blocks + 1]
+        bf.seg2 = (G1Xyzz*)get_scratch(c, "msm_seg2", ((size_t)pl.nwin * 24 * 33 + 2) * sizeof(G1Xyzz));   // [sets][jobs][blocks + 1]
     }
     bf.wins = (G1Xyzz*)get_scratch(c, "msm_wins", (size_t)2 * MSM_MAX_WINDOWS * sizeof(G1Xyzz));
     bf.count = (uint32_t*)get_scratch(c, "msm_count", 64);
@@ -289,39 +317,21 @@ static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBa
     const uint32_t *sorted_keys = nullptr, *sorted_vals = nullptr;
     std::unique_ptr<StageTimer> tmp(slot == 0 ? new StageTimer(c, "msm") : nullptr);   // stage timing: slot 0 only
     struct { StageTimer* t; void mark(const char* n) { if (t) t->mark(n); } } tm{tmp.get()};
-    int rc = msm_launch_digits_sort(c, pl, bf, batch, montgomery, &sorted_keys, &sorted_vals, tmp.get());
+    rc = msm_launch_digits_sort(c, pl, bf, batch, montgomery, &sorted_keys, &sorted_vals, tmp.get());
     if (rc != SWB_OK) return rc;
     tm.mark("count");
-    // batch-affine pair sums first when buckets are well filled and the input is large enough to amortise the block-wide
-    // inversions (swb_msm_set_pair_sums: 0 never, 1 automatic, 2 always)
-    bf.pair_levels = 0;
-    {
-        const double per_bucket = pl.nb ? (double)pl.total / (double)pl.nb : 0.0;
-        int levels = 0;
-        if (c->msm_pair_policy >= 2) levels = c->msm_pair_policy - 1;                 // forced: policy - 1 levels
-        else if (c->msm_pair_policy == 1 && pl.total >= msm_pair_min_total()) {
-            // measured: +9 % at 2^24 points, +12 % at 2^26, a 1/8 bucket share of 2^26 (92 M pairs) +3-7 %; the batched and
-            // single MSMs of a 2^20-constraint prover (17-160 M pairs, 26-100 per bucket) 0.334 -> 0.327 s with tables and
-            // 0.402 -> 0.375 s without; below 2^24 pairs the fixed cost of the block-wide inversions loses (2^16
-            // constraints: 44 -> 51 ms with the threshold at 2^22)
-            // a level pays while most aligned blocks of 2^L positions still lie inside one bucket
-            while (levels < MSM_PAIR_MAX_LEVELS && per_bucket >= (double)(8u << levels)) levels++;
+    if (pl.pair_levels > 0) {
+        static const char* const tags[MSM_PAIR_MAX_LEVELS + 1] = {"", "msm_pair_r1", "msm_pair_r2", "msm_pair_r3", "msm_pair_r4"};
+        for (int l = 1; l <= pl.pair_levels; l++) {
+            const size_t slots = (pl.total + ((size_t)1 << l) - 1) >> l;
+            bf.pair_sums[l] = (Fq*)get_scratch(c, tags[l], slots * 2 * sizeof(Fq) + 64);
+            if (!bf.pair_sums[l]) return SWB_ENOMEM;
         }
-        if (levels > MSM_PAIR_MAX_LEVELS) levels = MSM_PAIR_MAX_LEVELS;
-        if (levels > 0 && pl.total >= 2) {
-            static const char* const tags[MSM_PAIR_MAX_LEVELS + 1] = {"", "msm_pair_r1", "msm_pair_r2", "msm_pair_r3", "msm_pair_r4"};
-            for (int l = 1; l <= levels; l++) {
-                const size_t slots = (pl.total + ((size_t)1 << l) - 1) >> l;
-                bf.pair_sums[l] = (Fq*)get_scratch(c, tags[l], slots * 2 * sizeof(Fq) + 64);
-                if (!bf.pair_sums[l]) return SWB_ENOMEM;
-            }
-            bf.pair_lvl = (uint8_t*)get_scratch(c, "msm_pair_lvl", (pl.total + 1) / 2 + 64);
-            if (!bf.pair_lvl) return SWB_ENOMEM;
-            rc = msm_launch_pair_sums(c, pl, bf.pair_sums, bf.pair_lvl, levels, sorted_keys, sorted_vals, bases->xy, tmp.get());
-            if (rc != SWB_OK) return rc;
-            bf.pair_levels = levels;
-            tm.mark("pair_sums");
-        }
+        bf.pair_lvl = (uint8_t*)get_scratch(c, "msm_pair_lvl", (pl.total + 1) / 2 + 64);
+        if (!bf.pair_lvl) return SWB_ENOMEM;
+        rc = msm_launch_pair_sums(c, pl, bf.pair_sums, bf.pair_lvl, pl.pair_levels, sorted_keys, sorted_vals, bases->xy, tmp.get());
+        if (rc != SWB_OK) return rc;
+        tm.mark("pair_sums");
     }
     rc = msm_launch_accumulate(c, pl, bf, sorted_keys, sorted_vals, bases->xy);
     if (rc != SWB_OK) return rc;
@@ -344,18 +354,18 @@ static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBa
         cudaMemcpyAsync(&np, bf.range_off + pl.nranges, 4, cudaMemcpyDeviceToHost, c->stream);
         cudaMemcpyAsync(&nheavy, bf.heavy, 4, cudaMemcpyDeviceToHost, c->stream);
         cudaStreamSynchronize(c->stream);
-        fprintf(stderr, "[swb trace] msm: n=%zu c=%d windows=%d buckets=%u range_len=%u ranges=%u partials=%u heavy_buckets=%u\n", n,
-                cb, nwin, pl.nb, pl.range_len, pl.nranges, np, nheavy);
+        fprintf(stderr, "[swb trace] msm: n=%zu c=%d windows=%d buckets=%u range_len=%u ranges=%u partials=%u heavy_buckets=%u\n", pl.n,
+                pl.cb, pl.nwin, pl.nb, pl.range_len, pl.nranges, np, nheavy);
     }
 
-    sl.nwin = nwin;
-    sl.cb = cb;
-    sl.batched = tables && batched;
+    sl.nwin = pl.nwin;
+    sl.cb = pl.cb;
+    sl.batched = batch.count > 1;
     sl.shard_rank = (int)pl.shard_rank;
     sl.shard_world = 1 << pl.shard_shift;
-    SWB_CUDA(c, cudaMemcpyAsync(sl.host_wins, bf.wins, sizeof(G1Xyzz) * nwin, cudaMemcpyDeviceToHost, c->stream));
+    SWB_CUDA(c, cudaMemcpyAsync(sl.host_wins, bf.wins, sizeof(G1Xyzz) * pl.nwin, cudaMemcpyDeviceToHost, c->stream));
     if (pl.shard_shift)
-        SWB_CUDA(c, cudaMemcpyAsync(static_cast<G1Xyzz*>(sl.host_wins) + nwin, bf.wins + MSM_MAX_WINDOWS, sizeof(G1Xyzz) * nwin,
+        SWB_CUDA(c, cudaMemcpyAsync(static_cast<G1Xyzz*>(sl.host_wins) + pl.nwin, bf.wins + MSM_MAX_WINDOWS, sizeof(G1Xyzz) * pl.nwin,
                                     cudaMemcpyDeviceToHost, c->stream));
     return SWB_OK;
 }
@@ -498,7 +508,7 @@ int swb_msm_g1_batch_dev(swb_ctx* c, const swb_bases* b, const size_t* offsets, 
     while (done < n_msms && rc == SWB_OK) {
         size_t cnt = n_msms - done < (size_t)MSM_MAX_BATCH ? n_msms - done : (size_t)MSM_MAX_BATCH;
         if (cnt < 2 || !msm_can_batch(c, b, cnt, ns + done)) break;
-        rc = msm_begin_batch(c, 0, b, cnt, offsets + done, scalars_dev + done, ns + done, montgomery);
+        rc = msm_begin_batch(c, 0, b, cnt, offsets + done, scalars_dev + done, ns + done, montgomery, ctx_bucket_shard(c));
         if (rc == SWB_OK) rc = msm_end(c, 0, outs + done);
         done += cnt;
     }
@@ -513,7 +523,7 @@ int swb_msm_g1_batch_dev(swb_ctx* c, const swb_bases* b, const size_t* offsets, 
             busy[slot] = false;
             if (rc != SWB_OK) break;
         }
-        rc = msm_begin(c, slot, b, offsets[i], scalars_dev[i], ns[i], montgomery);
+        rc = msm_begin(c, slot, b, offsets[i], scalars_dev[i], ns[i], montgomery, ctx_bucket_shard(c));
         if (rc == SWB_OK) { busy[slot] = true; pending[slot] = i; }
     }
     for (int slot = 1; slot < swb_ctx::MSM_SLOTS; slot++)
@@ -527,28 +537,12 @@ int swb_msm_g1_batch_dev(swb_ctx* c, const swb_bases* b, const size_t* offsets, 
 int swb_msm_g1(swb_ctx* c, const swb_bases* b, size_t offset, const swb_bigint256* scalars_host, size_t n,
                swb_g1_jacobian* out) {
     if (!c) return SWB_EARG;
-    SWB_REQUIRE(c, n == 0 || scalars_host != nullptr, "msm: NULL scalars");
-    void* d = nullptr;
-    if (n) {
-        SWB_CUDA(c, cudaSetDevice(c->device));
-        d = get_scratch(c, "msm_scalars", n * 32);
-        if (!d) return SWB_ENOMEM;
-        SWB_CUDA(c, cudaMemcpyAsync(d, scalars_host, n * 32, cudaMemcpyHostToDevice, c->stream));
-    }
-    return msm_run(c, b, offset, d, n, 0, out);
+    return msm_run_host(c, b, offset, scalars_host, n, 0, out);
 }
 
 int swb_msm_g1_fr(swb_ctx* c, const swb_bases* b, size_t offset, const swb_fr* scalars_host, size_t n, swb_g1_jacobian* out) {
     if (!c) return SWB_EARG;
-    SWB_REQUIRE(c, n == 0 || scalars_host != nullptr, "msm: NULL scalars");
-    void* d = nullptr;
-    if (n) {
-        SWB_CUDA(c, cudaSetDevice(c->device));
-        d = get_scratch(c, "msm_scalars", n * 32);
-        if (!d) return SWB_ENOMEM;
-        SWB_CUDA(c, cudaMemcpyAsync(d, scalars_host, n * 32, cudaMemcpyHostToDevice, c->stream));
-    }
-    return msm_run(c, b, offset, d, n, 1, out);
+    return msm_run_host(c, b, offset, scalars_host, n, 1, out);
 }
 
 int swb_g1_sum_jacobian(swb_ctx* c, const swb_g1_jacobian* pts, size_t n, swb_g1_jacobian* out) {

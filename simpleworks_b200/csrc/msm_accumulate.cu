@@ -179,9 +179,9 @@ __global__ void __launch_bounds__(128) k_msm_accumulate_paired(G1Xyzz* __restric
 int msm_launch_accumulate(swb_ctx* c, const MsmPlan& pl, const MsmBuffers& bf, const uint32_t* sorted_keys,
                           const uint32_t* sorted_vals, const Fq* bases) {
     if (pl.nranges == 0) return SWB_OK;      // a bucket shard that received no pairs
-    if (bf.pair_levels > 0) {
+    if (pl.pair_levels > 0) {
         PairLevels pv{};
-        for (int l = 1; l <= bf.pair_levels; l++) pv.R[l] = bf.pair_sums[l];
+        for (int l = 1; l <= pl.pair_levels; l++) pv.R[l] = bf.pair_sums[l];
         pv.lvl = bf.pair_lvl;
         k_msm_accumulate_paired<<<(pl.nranges + 127) / 128, 128, 0, c->stream>>>(bf.partial, bf.pkey, bf.range_off, sorted_keys,
                                                                                 sorted_vals, bases, pv, pl.total, pl.seg_len,

@@ -7,6 +7,11 @@ namespace swb {
 
 constexpr int MSM_MAX_WINDOWS = 128;
 constexpr int MSM_PAIR_MAX_LEVELS = 4;   // summed blocks of up to 16 positions (the shortest accumulation range)
+// sorted pairs from which batch-affine pair sums run automatically.  Measured: +9 % at 2^24 points, +12 % at 2^26, a 1/8
+// bucket share of 2^26 (92 M pairs) +3-7 %; the batched and single MSMs of a 2^20-constraint prover (17-160 M pairs, 26-100
+// per bucket) 0.334 -> 0.327 s with tables and 0.402 -> 0.375 s without; below 2^24 pairs the fixed cost of the block-wide
+// inversions loses (2^16 constraints: 44 -> 51 ms with the threshold at 2^22)
+constexpr size_t MSM_PAIR_MIN_PAIRS = (size_t)1 << 24;
 // block size of the heavy-bucket gather: a bucket that holds a large share of all points (scalars equal to
 // one, top window) has one partial sum per range, i.e. up to ~10^5 of them, summed by one block
 constexpr int MSM_HEAVY_THREADS = 256;
@@ -52,6 +57,7 @@ struct MsmPlan {
     size_t tab_stride;   // records per table level (0 = plain path)
     uint32_t B;          // buckets per set that this call fills: 2^(cb-1), or that divided by the bucket-shard world
     uint32_t shard_rank, shard_shift;   // bucket sharding: ours are the buckets b with b mod 2^shift == rank, stored at b >> shift
+    bool idle;           // bucket shard with too few buckets to split: rank 0 computes all of it, this rank contributes the identity
     bool compact;        // table path under bucket sharding: only the pairs of our buckets are kept (total is then
                          // known after the digits kernel)
     uint32_t nb;         // total buckets = nwin * B
@@ -61,7 +67,12 @@ struct MsmPlan {
     uint32_t range_len;  // sorted positions per accumulation thread
     uint32_t nranges;    // ceil(total / range_len)
     uint32_t pcap;       // capacity of the partial-sum list (nranges + nb)
+    int pair_levels;     // levels of batch-affine pair sums in front of the accumulation (0 = none)
 };
+
+// plans what depends on the number of sorted pairs (pl.total): the accumulation ranges and the pair-sum levels.  msm_plan
+// calls it, and msm_launch_digits_sort again once a compacting digits kernel has counted the pairs it kept.
+void msm_plan_pairs(const swb_ctx* c, MsmPlan& pl);
 
 struct MsmBuffers {
     uint32_t* keys;      // [2][msm_alt_offset(total)]
@@ -76,7 +87,6 @@ struct MsmBuffers {
     G1Xyzz* seg2;        // per-job partial sums and values of the bucket reduction
     G1Xyzz* wins;        // [2][MSM_MAX_WINDOWS]: weighted sums sum_k (k+1) B_k, then plain sums sum_k B_k (bucket shards)
     uint32_t* count;     // [1] pairs kept by the compacting digits kernel
-    int pair_levels;                           // levels of batch-affine pair sums in front of the accumulation (0 = none)
     Fq* pair_sums[MSM_PAIR_MAX_LEVELS + 1];    // [l]: ceil(total / 2^l) slots of two field elements (msm_pairs.cu)
     uint8_t* pair_lvl;                         // [ceil(total / 2)] level map read by k_msm_accumulate_paired
 };

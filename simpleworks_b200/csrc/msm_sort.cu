@@ -80,128 +80,14 @@ __device__ __forceinline__ bool digits_load(const MsmBatch& batch, size_t i, siz
 // writes its pairs there -- the arrays the sort sees shrink with the number of ranks.
 // A batch (several scalar vectors over one bases handle, table path only) gives vector k its own bucket set: its keys are
 // k * Bloc + bucket, its points start at record batch.offset[k]; the marker is the number of buckets of the whole batch.
-template <bool COMPACT>
-__global__ void __launch_bounds__(256) k_msm_digits(uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
-                                                     MsmBatch batch, size_t n, int c, int nwin,
-                                                     int montgomery, size_t tab_stride, uint32_t rank, uint32_t shift, uint32_t Bloc,
-                                                     uint32_t* __restrict__ count) {
-    const uint32_t marker = Bloc * batch.count;
-    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const size_t stride = (size_t)gridDim.x * blockDim.x;
-    const uint32_t B = 1u << (c - 1);
-    __shared__ uint32_t s_cnt, s_base;
-    // compaction is a block-wide step, so every thread of the block runs the same number of rounds
-    const size_t rounds = (n + stride - 1) / stride;
-    for (size_t round = 0; round < rounds; round++, i += stride) {
-        Fr s;
-        uint32_t flip, key0;
-        size_t rec;
-        const bool live = digits_load(batch, i, n, montgomery, tab_stride, Bloc, s, flip, key0, rec);
-        // Signed digits, lowest window first: the scalar sits in a 256-bit shift register (eight funnel shifts per
-        // window), so no limb is ever indexed by a run-time value.  next_digit returns |digit| and sets neg / carry.
-        const uint32_t cmask = (1u << c) - 1u;
-        auto next_digit = [&](uint32_t (&t)[8], uint32_t& carry, uint32_t& neg) -> uint32_t {
-            uint32_t v = (t[0] & cmask) + carry;
-#pragma unroll
-            for (int k = 0; k < 7; k++) t[k] = __funnelshift_r(t[k], t[k + 1], (uint32_t)c);
-            t[7] >>= c;
-            neg = v > B ? 1u : 0u;
-            if (neg) v = (1u << c) - v;
-            carry = neg;
-            return v;
-        };
-        const uint32_t smask = (1u << shift) - 1u;
-        if (!COMPACT) {
-            if (live) {
-                uint32_t t[8], carry = 0, neg;
-#pragma unroll
-                for (int k = 0; k < 8; k++) t[k] = s.l[k];
-                for (int w = 0; w < nwin; w++) {
-                    const uint32_t v = next_digit(t, carry, neg);
-                    const uint32_t key = (v && ((v - 1) & smask) == rank) ? key0 + ((v - 1) >> shift) : marker;
-                    keys[(size_t)w * n + i] = key;
-                    vals[(size_t)w * n + i] = (uint32_t)(tab_stride ? (size_t)w * tab_stride + rec : rec) | ((neg ^ flip) << 31);
-                }
-            }
-            continue;
-        }
-        // count, reserve (one global atomic per block and round), write.  The first walk notes WHICH windows are ours
-        // (a bit mask); a warp's pairs are laid out window by window, so that the lanes keeping window w write
-        // neighbouring slots (one ballot per window gives a lane its place) instead of every lane its own run.
-        if (threadIdx.x == 0) s_cnt = 0;
-        __syncthreads();
-        uint32_t keep = 0;                                 // table levels <= 32
-        if (live) {
-            uint32_t t[8], carry = 0, neg;
-#pragma unroll
-            for (int k = 0; k < 8; k++) t[k] = s.l[k];
-            for (int w = 0; w < nwin; w++) {
-                const uint32_t v = next_digit(t, carry, neg);
-                if (v && ((v - 1) & smask) == rank) keep |= 1u << w;
-            }
-        }
-        const uint32_t lane = threadIdx.x & 31u;
-        uint32_t warp_total = 0;
-        for (int w = 0; w < nwin; w++) warp_total += (uint32_t)__popc(__ballot_sync(0xffffffffu, (keep >> w) & 1u));
-        uint32_t warp_base = 0;
-        if (lane == 0 && warp_total) warp_base = atomicAdd(&s_cnt, warp_total);
-        warp_base = __shfl_sync(0xffffffffu, warp_base, 0);
-        __syncthreads();
-        if (threadIdx.x == 0) s_base = s_cnt ? atomicAdd(count, s_cnt) : 0u;
-        __syncthreads();
-        if (warp_total == 0) continue;                     // warp-uniform
-        uint32_t seg = s_base + warp_base;
-        const uint32_t below = (1u << lane) - 1u;
-        uint32_t t[8], carry = 0, neg;
-#pragma unroll
-        for (int k = 0; k < 8; k++) t[k] = s.l[k];
-        for (int w = 0; w < nwin; w++) {
-            const uint32_t v = next_digit(t, carry, neg);
-            const uint32_t mine = (keep >> w) & 1u;
-            const uint32_t who = __ballot_sync(0xffffffffu, mine);
-            if (mine) {
-                const uint32_t at = seg + (uint32_t)__popc(who & below);
-                keys[at] = key0 + ((v - 1) >> shift);
-                vals[at] = (uint32_t)((size_t)w * tab_stride + rec) | ((neg ^ flip) << 31);
-            }
-            seg += (uint32_t)__popc(who);
-        }
-    }
-}
-
-// ---- 3. number of runs of equal (valid) keys inside each range of `len` sorted positions -----
-// Range r owns sorted positions [r*len, (r+1)*len), len a power of two >= 16.  Position p belongs
-// to window p / n; its global bucket id is (p / n) * B + key, and key == B marks a zero digit (the
-// tail of every window's segment).  A run is a maximal stretch of one global bucket id inside the
-// range; k_msm_accumulate emits exactly one partial sum per run, so the exclusive scan of these
-// counts is where each range writes.  One thread per position (coalesced), one atomic per half warp.
-__global__ void __launch_bounds__(256) k_msm_range_count(uint32_t* __restrict__ cnt, const uint32_t* __restrict__ keys,
-                                                          size_t total, size_t n, uint32_t B, uint32_t len) {
-    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    bool starts = false;
-    if (p < total) {
-        const uint32_t k = keys[p];
-        if (k < B) {
-            starts = true;                                     // first position of a range or window, or after a zero digit
-            if (p % len != 0 && p % n != 0) starts = keys[p - 1] != k;
-        }
-    }
-    const uint32_t ballot = __ballot_sync(0xffffffffu, starts);
-    const uint32_t lane = threadIdx.x & 31;
-    if ((lane & 15) == 0 && p < total) {
-        const uint32_t c = __popc(ballot & (lane ? 0xffff0000u : 0x0000ffffu));
-        if (c) atomicAdd(&cnt[p / len], c);
-    }
-}
-
-// ---- window width known at compile time ---------------------------------------------------------------------
-// Every window position is then a constant: a digit costs two shifts instead of a walk of the whole scalar through a
-// shift register, and the digits and warp votes of all windows stay in registers, so nothing is computed twice
-// (ncu, 2^26 scalars, 1/8 bucket share: the generic kernel executes ~950 warp instructions per 32 scalars and is
-// issue-bound at 2.4-2.6 ms; this one 1.9 ms).  Measured and dropped: splitting the compaction into two
-// barrier-free kernels (count per warp, scan, place) -- 420 + 665 instructions per 32 scalars, 2.7 ms.
+// The window width C is a template parameter, so every window position is a constant: a digit costs two shifts, and the
+// digits and warp votes of all windows stay in registers, so nothing is computed twice (ncu, 2^26 scalars, 1/8 bucket
+// share: with the width known only at run time, the scalar walked through a 256-bit shift register, the kernel executed
+// ~950 warp instructions per 32 scalars and was issue-bound at 2.4-2.6 ms; with it fixed, 1.9 ms).  Measured and dropped:
+// splitting the compaction into two barrier-free kernels (count per warp, scan, place) -- 420 + 665 instructions per 32
+// scalars, 2.7 ms.
 template <int C>
-struct DigitsFixed {
+struct Digits {
     static constexpr int NW = (254 + C - 1) / C;          // nwin <= NW
     static constexpr uint32_t CM = (1u << C) - 1u, B = 1u << (C - 1);
     // |digit| with the sign (already combined with `flip`) in bit 31; 0: nothing to add
@@ -225,11 +111,11 @@ struct DigitsFixed {
 };
 
 template <bool COMPACT, int C>
-__global__ void __launch_bounds__(256) k_msm_digits_fixed(uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
-                                                           MsmBatch batch, size_t n, int nwin,
-                                                           int montgomery, size_t tab_stride, uint32_t rank, uint32_t shift, uint32_t Bloc,
-                                                           uint32_t* __restrict__ count) {
-    using D = DigitsFixed<C>;
+__global__ void __launch_bounds__(256) k_msm_digits(uint32_t* __restrict__ keys, uint32_t* __restrict__ vals,
+                                                     MsmBatch batch, size_t n, int nwin,
+                                                     int montgomery, size_t tab_stride, uint32_t rank, uint32_t shift, uint32_t Bloc,
+                                                     uint32_t* __restrict__ count) {
+    using D = Digits<C>;
     const uint32_t marker = Bloc * batch.count;
     const uint32_t smask = (1u << shift) - 1u;
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -289,34 +175,61 @@ __global__ void __launch_bounds__(256) k_msm_digits_fixed(uint32_t* __restrict__
     }
 }
 
-// false: no kernel for this width (narrow windows of small inputs go to the generic kernel)
-template <bool COMPACT>
-static bool msm_launch_digits_fixed(int cb, unsigned blocks, cudaStream_t st, uint32_t* keys, uint32_t* vals, const MsmBatch& batch,
-                                    size_t n, int nwin, int montgomery, size_t tab_stride, uint32_t rank, uint32_t shift,
-                                    uint32_t Bloc, uint32_t* count) {
-    switch (cb) {
-#define SWB_DIGITS_CASE(CB)                                                                                              \
-    case CB:                                                                                                             \
-        if (nwin > DigitsFixed<CB>::NW) return false;                                                                    \
-        k_msm_digits_fixed<COMPACT, CB><<<blocks, 256, 0, st>>>(keys, vals, batch, n, nwin, montgomery, tab_stride, rank, \
-                                                                shift, Bloc, count);                                     \
-        return true;
-        SWB_DIGITS_CASE(12) SWB_DIGITS_CASE(13) SWB_DIGITS_CASE(14) SWB_DIGITS_CASE(15) SWB_DIGITS_CASE(16)
-        SWB_DIGITS_CASE(17) SWB_DIGITS_CASE(18) SWB_DIGITS_CASE(19) SWB_DIGITS_CASE(20) SWB_DIGITS_CASE(21)
-        SWB_DIGITS_CASE(22) SWB_DIGITS_CASE(23) SWB_DIGITS_CASE(24)
+// launches k_msm_digits<pl.compact, pl.cb>.  Every width the plan can choose has one: c in [2, 24] on the plain path
+// (swb_msm_set_window_bits, pick_window), c in [8, 24] over tables (swb_bases_precompute), and only tables compact.
+template <int C>
+static int msm_launch_digits(swb_ctx* c, const MsmPlan& pl, const MsmBuffers& bf, const MsmBatch& batch, int montgomery,
+                             unsigned blocks) {
+    if (pl.ndig > Digits<C>::NW) return set_err(c, SWB_EINTERNAL, "msm: %d digits of %d bits exceed the digits kernel", pl.ndig, C);
+    if (!pl.compact)
+        k_msm_digits<false, C><<<blocks, 256, 0, c->stream>>>(bf.keys, bf.vals, batch, pl.n, pl.ndig, montgomery, pl.tab_stride,
+                                                               pl.shard_rank, pl.shard_shift, pl.B, nullptr);
+    else if constexpr (C >= 8)
+        k_msm_digits<true, C><<<blocks, 256, 0, c->stream>>>(bf.keys, bf.vals, batch, pl.n, pl.ndig, montgomery, pl.tab_stride,
+                                                              pl.shard_rank, pl.shard_shift, pl.B, bf.count);
+    else
+        return set_err(c, SWB_EINTERNAL, "msm: no compacting digits kernel for c = %d (window tables have c >= 8)", C);
+    SWB_LAUNCH_CHECK(c, "k_msm_digits");
+    return SWB_OK;
+}
+
+static int msm_launch_digits(swb_ctx* c, const MsmPlan& pl, const MsmBuffers& bf, const MsmBatch& batch, int montgomery,
+                             unsigned blocks) {
+    switch (pl.cb) {
+#define SWB_DIGITS_CASE(CB) \
+    case CB: return msm_launch_digits<CB>(c, pl, bf, batch, montgomery, blocks);
+        SWB_DIGITS_CASE(2) SWB_DIGITS_CASE(3) SWB_DIGITS_CASE(4) SWB_DIGITS_CASE(5) SWB_DIGITS_CASE(6) SWB_DIGITS_CASE(7)
+        SWB_DIGITS_CASE(8) SWB_DIGITS_CASE(9) SWB_DIGITS_CASE(10) SWB_DIGITS_CASE(11) SWB_DIGITS_CASE(12) SWB_DIGITS_CASE(13)
+        SWB_DIGITS_CASE(14) SWB_DIGITS_CASE(15) SWB_DIGITS_CASE(16) SWB_DIGITS_CASE(17) SWB_DIGITS_CASE(18) SWB_DIGITS_CASE(19)
+        SWB_DIGITS_CASE(20) SWB_DIGITS_CASE(21) SWB_DIGITS_CASE(22) SWB_DIGITS_CASE(23) SWB_DIGITS_CASE(24)
 #undef SWB_DIGITS_CASE
-        default: return false;
+        default: return set_err(c, SWB_EINTERNAL, "msm: no digits kernel for c = %d", pl.cb);
     }
 }
 
-// fills in what is only known after the digits kernel under compaction: total, seg_len, ranges
-static void msm_plan_ranges(swb_ctx* c, MsmPlan& pl) {
-    // enough threads to fill the GPU (>= ~512 per SM) but at most 128 additions each
-    size_t want = pl.total / ((size_t)c->sm_count * 512);
-    uint32_t len = 16;
-    while (len < 128 && len < want) len <<= 1;
-    pl.range_len = len;
-    pl.nranges = (uint32_t)((pl.total + len - 1) / len);
+// ---- 3. number of runs of equal (valid) keys inside each range of `len` sorted positions -----
+// Range r owns sorted positions [r*len, (r+1)*len), len a power of two >= 16.  Position p belongs
+// to window p / n; its global bucket id is (p / n) * B + key, and key == B marks a zero digit (the
+// tail of every window's segment).  A run is a maximal stretch of one global bucket id inside the
+// range; k_msm_accumulate emits exactly one partial sum per run, so the exclusive scan of these
+// counts is where each range writes.  One thread per position (coalesced), one atomic per half warp.
+__global__ void __launch_bounds__(256) k_msm_range_count(uint32_t* __restrict__ cnt, const uint32_t* __restrict__ keys,
+                                                          size_t total, size_t n, uint32_t B, uint32_t len) {
+    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool starts = false;
+    if (p < total) {
+        const uint32_t k = keys[p];
+        if (k < B) {
+            starts = true;                                     // first position of a range or window, or after a zero digit
+            if (p % len != 0 && p % n != 0) starts = keys[p - 1] != k;
+        }
+    }
+    const uint32_t ballot = __ballot_sync(0xffffffffu, starts);
+    const uint32_t lane = threadIdx.x & 31;
+    if ((lane & 15) == 0 && p < total) {
+        const uint32_t c = __popc(ballot & (lane ? 0xffff0000u : 0x0000ffffu));
+        if (c) atomicAdd(&cnt[p / len], c);
+    }
 }
 
 int msm_launch_digits_sort(swb_ctx* c, MsmPlan& pl, const MsmBuffers& bf, const MsmBatch& batch, int montgomery,
@@ -325,26 +238,17 @@ int msm_launch_digits_sort(swb_ctx* c, MsmPlan& pl, const MsmBuffers& bf, const 
         size_t blocks = (pl.n + 255) / 256;
         size_t cap = (size_t)c->sm_count * 8;
         if (blocks > cap) blocks = cap;
+        if (pl.compact) SWB_CUDA(c, cudaMemsetAsync(bf.count, 0, sizeof(uint32_t), c->stream));
+        int rc = msm_launch_digits(c, pl, bf, batch, montgomery, (unsigned)blocks);
+        if (rc != SWB_OK) return rc;
         if (pl.compact) {
-            SWB_CUDA(c, cudaMemsetAsync(bf.count, 0, sizeof(uint32_t), c->stream));
-            if (!msm_launch_digits_fixed<true>(pl.cb, (unsigned)blocks, c->stream, bf.keys, bf.vals, batch, pl.n, pl.ndig, montgomery,
-                                               pl.tab_stride, pl.shard_rank, pl.shard_shift, pl.B, bf.count))
-                k_msm_digits<true><<<(unsigned)blocks, 256, 0, c->stream>>>(bf.keys, bf.vals, batch, pl.n, pl.cb,
-                                                                             pl.ndig, montgomery, pl.tab_stride, pl.shard_rank, pl.shard_shift, pl.B, bf.count);
-            SWB_LAUNCH_CHECK(c, "k_msm_digits");
             // the number of pairs that fell into our buckets sizes everything downstream
             uint32_t kept = 0;
             SWB_CUDA(c, cudaMemcpyAsync(&kept, bf.count, sizeof kept, cudaMemcpyDeviceToHost, c->stream));
             SWB_CUDA(c, cudaStreamSynchronize(c->stream));
             pl.total = kept;
             pl.seg_len = kept;
-            msm_plan_ranges(c, pl);
-        } else {
-            if (!msm_launch_digits_fixed<false>(pl.cb, (unsigned)blocks, c->stream, bf.keys, bf.vals, batch, pl.n, pl.ndig, montgomery,
-                                                pl.tab_stride, pl.shard_rank, pl.shard_shift, pl.B, nullptr))
-                k_msm_digits<false><<<(unsigned)blocks, 256, 0, c->stream>>>(bf.keys, bf.vals, batch, pl.n, pl.cb,
-                                                                              pl.ndig, montgomery, pl.tab_stride, pl.shard_rank, pl.shard_shift, pl.B, nullptr);
-            SWB_LAUNCH_CHECK(c, "k_msm_digits");
+            msm_plan_pairs(c, pl);
         }
     }
     if (tm) tm->mark("digits");

@@ -1,9 +1,8 @@
 """The MSM's digit kernels at every window width, alone and under bucket shards, against the exact reference
 of oracle/commit_ref.py: over bases P_i = beta^i * G an MSM equals (sum_i s_i beta^i) * G.
 
-Plain path: c = 2..24 (k_msm_digits below 12, k_msm_digits_fixed<false, c> from 12 on).  Table path: c = 8..24
-(the compacting kernel k_msm_digits_fixed<true, c> runs under bucket shards from c = 12 on, the generic
-k_msm_digits<true> below).  The scalars of width c put every c-bit window on a digit boundary (0, 1, B - 1, B,
+Plain path: c = 2..24 (k_msm_digits<false, c>).  Table path: c = 8..24 (the compacting kernel k_msm_digits<true, c>
+runs under bucket shards).  The scalars of width c put every c-bit window on a digit boundary (0, 1, B - 1, B,
 B + 1, 2^c - 1 with B = 2^(c - 1)), so that carries, the sign flip at B and the top window all occur; their
 negations r - s take the table path's flip.  Bucket shards are run rank by rank on one GPU: a share does not
 depend on where it is computed, and the shares must add up to the reference."""
@@ -182,7 +181,7 @@ def test_heavy_bucket_chunks(be, c):
 
 @pytest.mark.parametrize("c", [11, 17, 23])
 def test_msm_batch_under_shards(be, c):
-    """swb_msm_g1_batch_dev over tables (one bucket set per vector; c = 11: generic kernel) with mixed sizes,
+    """swb_msm_g1_batch_dev over tables (one bucket set per vector) with mixed sizes,
     empty and single vectors and offsets: every vector's shares add up to its single-call result and to the
     reference, in both scalar forms"""
     n = 12000

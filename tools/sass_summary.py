@@ -10,7 +10,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "simpleworks_b200", "_build")
-KERNELS = {"msm_pairs.o": ["k_pair_bwd", "k_pair_fwd", "k_pair_inv"], "msm_accumulate.o": ["k_msm_accumulate"], "ntt.o": ["k_ntt_pass"], "msm_sort.o": ["k_msm_digits_fixedILb1ELi23", "k_msm_digits_fixedILb0ELi20", "k_msm_digitsILb1"],
+KERNELS = {"msm_pairs.o": ["k_pair_bwd", "k_pair_fwd", "k_pair_inv"], "msm_accumulate.o": ["k_msm_accumulate"], "ntt.o": ["k_ntt_pass"], "msm_sort.o": ["k_msm_digitsILb1ELi23E", "k_msm_digitsILb0ELi20E"],
            "vec.o": ["k_mul_peak", "k_fq_mul", "k_fr_mul"]}
 
 

@@ -216,6 +216,7 @@ int  swb_ntt_fr_batch_dev(swb_ctx*, swb_fr* inout_dev, uint32_t log_n, size_t ba
  *   swb_marlin_index             generate_proving_and_verifying_keys               mod.rs:88-94
  *   swb_marlin_prove             generate_proof + serialize_proof    mod.rs:70-77, serialization.rs:5
  *   swb_marlin_verify            deserialize_proof + verify_proof    serialization.rs:14, mod.rs:79-86
+ *   swb_marlin_verify_batch      the same for many proofs at once (SimpleMerkleTree::verify, a ledger's block)
  * swb_r1cs is what a ConstraintSystemRef exposes (to_matrices() + assignments; mod.rs:16): columns
  * are instance variables first (column 0 = the constant one), then witnesses.  public_inputs for
  * verify exclude the leading one, as in simple_merkle_tree.rs:133-143.
@@ -286,6 +287,20 @@ int  swb_marlin_prove(swb_ctx*, const swb_pk*, const swb_r1cs* cs_with_assignmen
  * seed.  ctx may be NULL: verification is host arithmetic (BLS12-377 pairing), no GPU involved. */
 int  swb_marlin_verify(swb_ctx*, const swb_vk*, const swb_fr* public_inputs, size_t n, const uint8_t* proof, size_t len,
                        swb_rng*, int* ok);
+/* Verifies n proofs in one call: ok[i] = the verdict of swb_marlin_verify(ctx, vks[i], public_inputs[i], n_inputs[i],
+ * proofs[i], lens[i]) for every i < n, except with negligible probability; proofs and keys as in swb_marlin_verify.
+ * A malformed proof, a point off the curve or outside G1, a wrong input count or a missing shift power gives ok[i] = 0,
+ * not an error.  The keys may all be the same or all differ; proofs whose keys share (h, beta_h) -- keys indexed from
+ * one SRS -- are checked together by ONE pairing equation, the proofs weighted by independent secret 128-bit scalars;
+ * when it fails, halves of the proofs are checked the same way until each invalid proof is found.  The context is
+ * required: the proofs' G1 points are decoded and summed (MSM) on its GPU; the context's bucket shard does not apply.
+ * rng as in swb_marlin_verify (NULL: OS entropy, never a fixed seed).  The call draws 2 n u128 from it: for each proof
+ * in index order, whether or not it parses, its weight and then the scalar that folds its two openings, so a seeded
+ * rng gives reproducible verdicts.  Returns non-zero only for bad arguments, CUDA failures or a missing entropy
+ * source, and then every ok[i] is 0; n = 0 returns SWB_OK.  With swb_profile_enable the stage times (parse, decode,
+ * transcripts, msm, pairing, bisect) are kept for swb_profile_last. */
+int  swb_marlin_verify_batch(swb_ctx*, size_t n, const swb_vk* const* vks, const swb_fr* const* public_inputs,
+                             const size_t* n_inputs, const uint8_t* const* proofs, const size_t* lens, swb_rng*, int* ok);
 void swb_bytes_free(uint8_t*);
 /* serialize_verifying_key / deserialize_verifying_key (reference src/marlin/serialization.rs:19-31);
  * NULL on malformed input. */

@@ -31,7 +31,7 @@ SYMBOLS = [
     "swb_r1cs_new", "swb_r1cs_builtin", "swb_r1cs_add_constraint", "swb_r1cs_set_assignment", "swb_r1cs_is_satisfied",
     "swb_r1cs_free",
     "swb_marlin_profile_enable", "swb_marlin_last_phases", "swb_marlin_universal_setup", "swb_srs_max_degree", "swb_srs_set_tune_after", "swb_srs_table_info", "swb_srs_free", "swb_marlin_index", "swb_pk_free", "swb_vk_free",
-    "swb_marlin_prove", "swb_marlin_verify", "swb_bytes_free",
+    "swb_marlin_prove", "swb_marlin_verify", "swb_marlin_verify_batch", "swb_bytes_free",
     "swb_vk_serialize", "swb_vk_deserialize", "swb_proof_deserialize", "swb_proof_serialize", "swb_proof_free", "swb_marlin_verify_proof", "swb_pk_serialize", "swb_pk_deserialize", "swb_r1cs_read", "swb_r1cs_write",
 ]
 
@@ -114,6 +114,7 @@ def load() -> ctypes.CDLL:
         "swb_vk_free": (None, [vp]),
         "swb_marlin_prove": (i32, [vp, vp, vp, vp, ctypes.POINTER(ctypes.POINTER(ctypes.c_uint8)), ctypes.POINTER(sz)]),
         "swb_marlin_verify": (i32, [vp, vp, vp, sz, ctypes.c_char_p, sz, vp, ctypes.POINTER(i32)]),
+        "swb_marlin_verify_batch": (i32, [vp, sz, vp, vp, vp, vp, vp, vp, ctypes.POINTER(i32)]),
         "swb_bytes_free": (None, [ctypes.POINTER(ctypes.c_uint8)]),
         "swb_vk_serialize": (i32, [vp, ctypes.POINTER(ctypes.POINTER(ctypes.c_uint8)), ctypes.POINTER(sz)]),
         "swb_vk_deserialize": (vp, [ctypes.c_char_p, sz]),

@@ -613,3 +613,25 @@ class Marlin:
         self.be._check(self._lib.swb_marlin_verify(self.be._h, vk, pi.ctypes.data, pi.shape[0], proof, len(proof),
                                                    rng._h if rng else None, ctypes.byref(ok)))
         return bool(ok.value)
+
+    def verify_proofs(self, vks, public_inputs, proofs, rng: "Rng | None" = None) -> list:
+        """[verify_proof(vks[i], public_inputs[i], proofs[i]) for every i] in one call (swb_marlin_verify_batch): the
+        proofs' points are decoded and summed on the GPU, and proofs of keys from one SRS share one pairing check.  A
+        single key is used for every proof.  The call draws two u128 per proof from rng (None: OS entropy)."""
+        n = len(proofs)
+        if not isinstance(vks, (list, tuple)):
+            vks = [vks] * n
+        if len(vks) != n or len(public_inputs) != n:
+            raise ValueError("verify_proofs: one key (or a single key) and one public-input array per proof")
+        pis = [np.ascontiguousarray(p, dtype=np.uint64).reshape(-1, 4) for p in public_inputs]
+        proofs = [bytes(p) for p in proofs]
+        vp = ctypes.c_void_p
+        arr_vk = (vp * max(n, 1))(*[v.value if isinstance(v, ctypes.c_void_p) else v for v in vks])
+        arr_pi = (vp * max(n, 1))(*[p.ctypes.data for p in pis])
+        arr_ni = (ctypes.c_size_t * max(n, 1))(*[p.shape[0] for p in pis])
+        arr_pr = (ctypes.c_char_p * max(n, 1))(*proofs)
+        arr_len = (ctypes.c_size_t * max(n, 1))(*[len(p) for p in proofs])
+        ok = (ctypes.c_int * max(n, 1))()
+        self.be._check(self._lib.swb_marlin_verify_batch(self.be._h, n, arr_vk, arr_pi, arr_ni, arr_pr, arr_len,
+                                                         rng._h if rng else None, ok))
+        return [bool(ok[i]) for i in range(n)]

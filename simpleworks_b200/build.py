@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "_build")
 SOURCES = ["ctx.cu", "vec.cu", "ntt.cu", "msm.cu", "msm_sort.cu", "radix_sort.cu", "msm_accumulate.cu", "msm_pairs.cu", "msm_reduce.cu", "fixed_base.cu", "polyops.cu", "marlin_ops.cu",
-           "marlin_abi.cu", "comm.cu", "index_ops.cu"]
+           "marlin_abi.cu", "comm.cu", "index_ops.cu", "verify_ops.cu"]
 LIB_SO = os.path.join(HERE, "libswb200.so")
 LIB_A = os.path.join(HERE, "libswb200.a")
 NVCC = os.environ.get("SWB_NVCC", "/usr/local/cuda/bin/nvcc")

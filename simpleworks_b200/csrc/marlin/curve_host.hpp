@@ -6,7 +6,7 @@
 #pragma once
 #include <vector>
 
-#include "../g1.cuh"
+#include "../g1_decode.cuh"
 #include "rng.hpp"
 
 namespace swb {
@@ -112,23 +112,19 @@ inline G1Xyzz g1_msm_host(const std::vector<std::pair<G1Point, Fr>>& terms) {
 
 // ---- Fq square roots ------------------------------------------------------------------------
 struct FqSqrtCtx {
-    uint32_t half[12];      // (q-1)/2
-    uint32_t t[12];         // (q-1) / 2^46
-    uint32_t t1h[12];       // (t+1)/2
-    Fq z;                   // 5^t: generator of the 2-Sylow subgroup (5 is a non-residue)
+    FqSqrtConsts k;         // what fq_sqrt_ts (g1_decode.cuh) needs: (t - 1) / 2 and z = 5^t, t = (q - 1) / 2^46
     FqSqrtCtx() {
-        uint32_t qm1[12];
+        uint32_t qm1[12], t[12];
         for (int i = 0; i < 12; i++) qm1[i] = FqParams::mod(i);
         qm1[0] -= 1;
-        shr(half, qm1, 1);
         shr(t, qm1, 46);
-        uint32_t tp1[12];
-        memcpy(tp1, t, sizeof tp1);
-        tp1[0] += 1;        // t is odd, no carry
-        shr(t1h, tp1, 1);
+        shr(k.tm1h, t, 1);      // t is odd: (t - 1) / 2 = t >> 1
+        k.tm1h_bits = 0;
+        for (int i = 0; i < 12 * 32; i++)
+            if ((k.tm1h[i >> 5] >> (i & 31)) & 1u) k.tm1h_bits = i + 1;
         Fq five = Fq::one();
         five = five + five + five + five + five;
-        z = pow(five, t);
+        k.z = pow(five, t);
     }
     static void shr(uint32_t* out, const uint32_t* in, int s) {
         for (int i = 0; i < 12; i++) {
@@ -137,60 +133,21 @@ struct FqSqrtCtx {
             out[i] = (uint32_t)(((hi << 32) | lo) >> b);
         }
     }
-    static Fq pow(const Fq& a, const uint32_t* e) {
-        Fq acc = Fq::one();
-        for (int i = 12 * 32 - 1; i >= 0; i--) {
-            acc = acc.sqr();
-            if ((e[i >> 5] >> (i & 31)) & 1u) acc = acc * a;
-        }
-        return acc;
-    }
-    bool is_square(const Fq& a) const { return a.is_zero() || pow(a, half) == Fq::one(); }
+    static Fq pow(const Fq& a, const uint32_t* e) { return fq_pow_bits(a, e, 12 * 32); }
     // Tonelli-Shanks; returns false when a is a non-residue
-    bool sqrt(const Fq& a, Fq* out) const {
-        if (a.is_zero()) { *out = a; return true; }
-        if (!is_square(a)) return false;
-        Fq x = pow(a, t1h);             // a^((t+1)/2)
-        Fq b = pow(a, t);               // a^t
-        Fq zz = z;
-        int m = 46;
-        while (!(b == Fq::one())) {
-            int k = 0;
-            Fq b2 = b;
-            while (!(b2 == Fq::one())) { b2 = b2.sqr(); k++; }
-            Fq w = zz;
-            for (int i = 0; i < m - k - 1; i++) w = w.sqr();
-            zz = w.sqr();
-            b = b * zz;
-            x = x * w;
-            m = k;
-        }
-        *out = x;
-        return true;
-    }
+    bool sqrt(const Fq& a, Fq* out) const { return fq_sqrt_ts(k, a, out); }
 };
 inline const FqSqrtCtx& fq_sqrt_ctx() {
     static const FqSqrtCtx c;
     return c;
 }
 
-// canonical integer comparison a > b (both Montgomery)
-inline bool fq_canonical_gt(const Fq& a, const Fq& b) {
-    Fq ca = a.to_canonical(), cb = b.to_canonical();
-    for (int i = 11; i >= 0; i--)
-        if (ca.l[i] != cb.l[i]) return ca.l[i] > cb.l[i];
-    return false;
-}
-
 // GroupAffine::get_point_from_x(x, greatest) for y^2 = x^3 + 1
 inline bool g1_point_from_x(const Fq& x, bool greatest, G1Point* out) {
-    Fq rhs = x.sqr() * x + Fq::one();
     Fq y;
-    if (!fq_sqrt_ctx().sqrt(rhs, &y)) return false;
-    Fq negy = y.neg();
-    const bool y_lt_negy = fq_canonical_gt(negy, y);
+    if (!g1_y_from_x(fq_sqrt_ctx().k, x, greatest, &y)) return false;
     out->x = x;
-    out->y = (y_lt_negy ^ greatest) ? y : negy;
+    out->y = y;
     out->infinity = false;
     return true;
 }
@@ -282,10 +239,9 @@ inline bool g1_in_subgroup_plain(const G1Point& p) {
     for (int i = 0; i < 8; i++) r[i] = FrParams::mod(i);
     return g1_mul_words(p, r, 8).is_identity();
 }
-// The same verdict from two 64-bit multiplications (Scott, "A note on group membership tests for G1, G2 and GT on BLS
-// pairing-friendly curves"; what ark-bls12-377 0.4 does): P is in G1 iff phi(P) = -[x^2]P, where phi(X, Y) = (beta X, Y)
-// is the curve's order-3 endomorphism and x the BLS parameter.  beta is the cube root of unity for which the identity
-// holds on the generator, found once; the self-test compares the verdicts of both tests on points inside and outside G1.
+// The same verdict from two 64-bit multiplications (g1_decode.cuh: g1_endo_holds).  beta is the cube root of unity
+// for which the identity holds on the generator, found once; the self-test compares the verdicts of both tests on
+// points inside and outside G1.
 struct G1EndoCtx {
     Fq beta;
     G1EndoCtx() {
@@ -305,45 +261,36 @@ struct G1EndoCtx {
         } while (b == Fq::one());
         const G1Point g = g1_generator();
         beta = b;
-        if (!holds(g, beta)) beta = b * b;
-    }
-    static G1Xyzz mul_x(const G1Point& p) {
-        const uint32_t xw[2] = {(uint32_t)SWB_BLS_X, (uint32_t)(SWB_BLS_X >> 32)};
-        return g1_mul_words(p, xw, 2);
-    }
-    static bool holds(const G1Point& p, const Fq& b) {
-        const G1Xyzz xp = mul_x(p);
-        if (xp.is_identity()) return false;
-        const G1Point xa = to_affine(xp);
-        if (xa.x == p.x && xa.y == p.y) return false;          // [x]P = P: not of order r
-        const G1Xyzz x2 = mul_x(xa);                            // [x^2]P must be (beta X, -Y)
-        if (x2.is_identity()) return false;
-        return x2.x == (b * p.x) * x2.zz && x2.y == p.y.neg() * x2.zzz;
+        if (!g1_endo_holds(g.x, g.y, beta)) beta = b * b;
     }
 };
+// the decoder's constants, computed once; the batch verifier passes the same values to its kernel
+inline const G1DecodeConsts& g1_decode_consts() {
+    static const G1DecodeConsts k = [] {
+        G1DecodeConsts r;
+        r.sq = fq_sqrt_ctx().k;
+        r.beta = G1EndoCtx().beta;
+        return r;
+    }();
+    return k;
+}
 inline bool g1_in_subgroup(const G1Point& p) {
     if (p.infinity) return true;
-    static const G1EndoCtx ctx;
-    return G1EndoCtx::holds(p, ctx.beta);
+    return g1_endo_holds(p.x, p.y, g1_decode_consts().beta);
 }
+// CanonicalDeserialize for GroupAffine (g1_decode.cuh); p advances by 48 bytes whatever the verdict
 inline bool get_g1_compressed(const uint8_t*& p, const uint8_t* end, G1Point* out) {
     if (end - p < 48) return false;
-    uint8_t buf[48];
-    memcpy(buf, p, 48);
-    const uint8_t flags = buf[47] & 0xC0;
-    buf[47] &= 0x3F;
+    uint32_t w[12];
+    for (int i = 0; i < 12; i++)
+        w[i] = (uint32_t)p[4 * i] | ((uint32_t)p[4 * i + 1] << 8) | ((uint32_t)p[4 * i + 2] << 16) | ((uint32_t)p[4 * i + 3] << 24);
     p += 48;
-    if (flags & 0x40) {
-        // the identity has one encoding: x = 0, no sign bit (stricter than upstream, which ignores x here)
-        if (flags & 0x80) return false;
-        for (int i = 0; i < 48; i++)
-            if (buf[i]) return false;
-        *out = G1Point::identity();
-        return true;
-    }
-    Fq x;
-    if (!fq_from_canonical_bytes(buf, &x)) return false;
-    return g1_point_from_x(x, (flags & 0x80) != 0, out) && g1_in_subgroup(*out);
+    Fq x, y;
+    if (g1_decode(g1_decode_consts(), w, &x, &y) != G1D_OK) return false;
+    out->x = x;
+    out->y = y;
+    out->infinity = x.is_zero() && y.is_zero();
+    return true;
 }
 
 }  // namespace marlin

@@ -675,7 +675,11 @@ struct Proof {
         out.push_back(0);                      // BatchLCProof.evals: None
         return out;
     }
-    static bool deserialize(const uint8_t* p, size_t len, Proof* out) {
+    static bool deserialize(const uint8_t* p, size_t len, Proof* out) { return deserialize(p, len, out, get_g1_compressed); }
+    // The same parser with the G1 points read by `get_point(p, end, G1Point* out)`, which has the signature and contract of
+    // get_g1_compressed: the batch verifier collects the encodings here and decodes them all at once on the GPU.
+    template <class PointReader>
+    static bool deserialize(const uint8_t* p, size_t len, Proof* out, PointReader&& get_point) {
         const uint8_t* end = p + len;
         auto get_u64 = [&](uint64_t* v) {
             if (end - p < 8) return false;
@@ -692,10 +696,10 @@ struct Proof {
             if (!get_u64(&m) || m > 64) return false;
             round.resize(m);
             for (auto& c : round) {
-                if (!get_g1_compressed(p, end, &c.comm)) return false;
+                if (!get_point(p, end, &c.comm)) return false;
                 if (p >= end) return false;
                 c.has_shifted = *p++ != 0;
-                if (c.has_shifted && !get_g1_compressed(p, end, &c.shifted)) return false;
+                if (c.has_shifted && !get_point(p, end, &c.shifted)) return false;
             }
         }
         if (!get_u64(&n) || n > 64) return false;
@@ -707,7 +711,7 @@ struct Proof {
         if (!get_u64(&n) || n > 8) return false;
         out->pc_proofs.resize(n);
         for (auto& pr : out->pc_proofs) {
-            if (!get_g1_compressed(p, end, &pr.w)) return false;
+            if (!get_point(p, end, &pr.w)) return false;
             if (p >= end) return false;
             pr.has_random_v = *p++ != 0;
             if (pr.has_random_v && !get_fr_canonical(p, end, &pr.random_v)) return false;
@@ -1050,12 +1054,28 @@ Proof prove(Engine& eng, const ProvingKey<Engine>& pk, const R1cs& cs, ChaChaRng
 // ------------------------------------------------------------------------------------------------
 // verify (Marlin::verify; SURVEY 3.4) -- public input WITHOUT the leading one, padded internally
 // ------------------------------------------------------------------------------------------------
-inline bool verify(const VerifyingKey& vk, const std::vector<Fr>& public_input_unpadded, const Proof& proof, ChaChaRng& rng) {
+// The structural checks that refuse a proof before its transcript is replayed
+inline bool verify_shape(const VerifyingKey& vk, size_t n_public_inputs, const Proof& proof) {
     if (proof.commitments.size() != 3 || proof.commitments[0].size() != 4 || proof.commitments[1].size() != 3 ||
         proof.commitments[2].size() != 2 || proof.evaluations.size() != 4 || proof.pc_proofs.size() != 2)
         return false;
+    if (Domain(n_public_inputs + 1).n != vk.info.num_instance || vk.index_comms.size() != 6) return false;
+    return proof.commitments[1][1].has_shifted && proof.commitments[2][0].has_shifted;     // g_1 and g_2 carry degree bounds
+}
+
+// kzg10::batch_check of one proof as two flat lists of (point, scalar) terms: the proof is valid iff
+//     e(sum c, h) * e(-sum w, beta_h) == 1.
+// The points are the proof's own and the key's (g, gamma_g, index commitments, shift powers); the pointers stay valid
+// while both live.  The opening at beta is weighted by w_beta, the one at gamma by w_gamma.
+struct CheckTerms {
+    std::vector<std::pair<const G1Point*, Fr>> c, w;
+};
+// Everything of verify up to the group arithmetic: shape checks, transcript replay, the linear combinations, the
+// terms.  false when the proof is refused on the way (shape, or a degree bound without a shift power in the key).
+inline bool verify_prepare(const VerifyingKey& vk, const std::vector<Fr>& public_input_unpadded, const Proof& proof,
+                           const Fr& w_beta, const Fr& w_gamma, CheckTerms* out) {
+    if (!verify_shape(vk, public_input_unpadded.size(), proof)) return false;
     Domain H(vk.info.num_constraints), K(vk.info.num_non_zero), X(public_input_unpadded.size() + 1);
-    if (X.n != vk.info.num_instance) return false;
     std::vector<Fr> public_input = public_input_unpadded;
     public_input.resize(X.n - 1, Fr::zero());
     FiatShamirRng fs;
@@ -1107,26 +1127,27 @@ inline bool verify(const VerifyingKey& vk, const std::vector<Fr>& public_input_u
     for (int i = 0; i < 4; i++) comm[r1[i]] = &proof.commitments[0][i];
     for (int i = 0; i < 3; i++) comm[r2[i]] = &proof.commitments[1][i];
     for (int i = 0; i < 2; i++) comm[r3[i]] = &proof.commitments[2][i];
-    if (vk.index_comms.size() != 6) return false;
     for (int i = 0; i < 6; i++) comm[ix[i]] = &vk.index_comms[i];
-    if (!comm["g_1"]->has_shifted || !comm["g_2"]->has_shifted) return false;
     struct Item { const Commitment* c; const LinComb* lc; Fr value; bool bounded; size_t bound; };
     // kzg10::batch_check: total_c = sum r_i (C_i - v_i g - v'_i gamma_g + z_i W_i), total_w = sum r_i W_i,
     // r_0 = 1, r_i = u128::rand(rng); accept iff e(total_c, h) == e(total_w, beta_h).
     // Every C_i is itself a combination of commitments (accumulate_commitments_and_values with the per-polynomial
     // opening challenge powers; the two virtual commitments are linear combinations of index and prover commitments),
-    // so both sums are flattened into ONE list of (point, scalar) terms each and evaluated by a single host MSM with
-    // shared doublings: the group elements are the ones the nested scalar multiplications would give.
-    std::vector<std::pair<G1Point, Fr>> terms_c, terms_w;
+    // so both sums are flattened into ONE list of (point, scalar) terms each: the group elements are the ones the
+    // nested scalar multiplications would give.
+    std::vector<std::pair<const G1Point*, Fr>>& terms_c = out->c;
+    std::vector<std::pair<const G1Point*, Fr>>& terms_w = out->w;
+    terms_c.clear();
+    terms_w.clear();
     bool ok = true;
     auto accumulate_point = [&](const std::vector<Item>& items, const Fr& z, const PcProof& pr, const Fr& randomizer) {
         Fr cv = Fr::zero(), chal = Fr::one();
         for (auto& it : items) {
             const Fr s = chal * randomizer;
             if (it.lc) {
-                for (auto& t : it.lc->terms) terms_c.push_back({comm.at(t.second)->comm, t.first * s});
+                for (auto& t : it.lc->terms) terms_c.push_back({&comm.at(t.second)->comm, t.first * s});
             } else {
-                terms_c.push_back({it.c->comm, s});
+                terms_c.push_back({&it.c->comm, s});
             }
             cv = cv + it.value * chal;
             chal = chal * ch.xi;
@@ -1134,27 +1155,41 @@ inline bool verify(const VerifyingKey& vk, const std::vector<Fr>& public_input_u
                 // (shifted_comm - value * beta^(D - bound) g) * next challenge power
                 const G1Point* sp = vk.shift_power(it.bound);
                 if (!sp) { ok = false; return; }
-                terms_c.push_back({it.c->shifted, chal * randomizer});
-                terms_c.push_back({*sp, (it.value * chal * randomizer).neg()});
+                terms_c.push_back({&it.c->shifted, chal * randomizer});
+                terms_c.push_back({sp, (it.value * chal * randomizer).neg()});
                 chal = chal * ch.xi;
             }
         }
-        terms_c.push_back({vk.g, (cv * randomizer).neg()});
-        if (pr.has_random_v) terms_c.push_back({vk.gamma_g, (pr.random_v * randomizer).neg()});
-        terms_c.push_back({pr.w, z * randomizer});
-        terms_w.push_back({pr.w, randomizer});
+        terms_c.push_back({&vk.g, (cv * randomizer).neg()});
+        if (pr.has_random_v) terms_c.push_back({&vk.gamma_g, (pr.random_v * randomizer).neg()});
+        terms_c.push_back({&pr.w, z * randomizer});
+        terms_w.push_back({&pr.w, randomizer});
     };
     std::vector<Item> at_beta = {{comm["g_1"], nullptr, in.g1_beta, true, H.n - 2},
                                  {nullptr, &outer, outer.constant.neg(), false, 0},
                                  {comm["t"], nullptr, in.t_beta, false, 0},
                                  {comm["z_b"], nullptr, in.zb_beta, false, 0}};
     std::vector<Item> at_gamma = {{comm["g_2"], nullptr, in.g2_gamma, true, K.n - 2}, {nullptr, &inner, inner.constant.neg(), false, 0}};
-    accumulate_point(at_beta, ch.beta, proof.pc_proofs[0], Fr::one());
+    accumulate_point(at_beta, ch.beta, proof.pc_proofs[0], w_beta);
+    if (ok) accumulate_point(at_gamma, ch.gamma, proof.pc_proofs[1], w_gamma);
+    return ok;
+}
+
+// The single-proof check: one u128 from rng folds the two openings (drawn once the proof has passed verify_shape), one
+// host MSM per side, one pairing product
+inline bool verify(const VerifyingKey& vk, const std::vector<Fr>& public_input_unpadded, const Proof& proof, ChaChaRng& rng) {
+    if (!verify_shape(vk, public_input_unpadded.size(), proof)) return false;
     uint64_t rw[2];
     rng.next_u128(rw);
-    accumulate_point(at_gamma, ch.gamma, proof.pc_proofs[1], fr_from_u128(rw));
-    if (!ok) return false;
-    const G1Xyzz total_c = g1_msm_host(terms_c), total_w = g1_msm_host(terms_w);
+    CheckTerms t;
+    if (!verify_prepare(vk, public_input_unpadded, proof, Fr::one(), fr_from_u128(rw), &t)) return false;
+    auto values = [](const std::vector<std::pair<const G1Point*, Fr>>& in) {
+        std::vector<std::pair<G1Point, Fr>> v;
+        v.reserve(in.size());
+        for (auto& t : in) v.push_back({*t.first, t.second});
+        return v;
+    };
+    const G1Xyzz total_c = g1_msm_host(values(t.c)), total_w = g1_msm_host(values(t.w));
     return pairing_product_is_one({{to_affine(total_c), vk.h}, {g1_neg(to_affine(total_w)), vk.beta_h}});
 }
 

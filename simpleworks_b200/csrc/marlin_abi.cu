@@ -7,6 +7,7 @@
 #include "index_ops.hpp"
 #include "marlin_ops.hpp"
 #include "polyops.hpp"
+#include "verify_ops.hpp"
 
 using namespace swb;
 using namespace swb::marlin;
@@ -741,6 +742,35 @@ int swb_marlin_verify(swb_ctx* c, const swb_vk* vk, const swb_fr* public_inputs,
     int rc = Api::verify(vk->h, (const uint64_t*)public_inputs, n, proof, len, rng ? &rng->h : nullptr, ok, &err);
     if (rc) return swb::set_err(c, SWB_EINTERNAL, "verify: %s", err.c_str());
     return SWB_OK;
+}
+int swb_marlin_verify_batch(swb_ctx* c, size_t n, const swb_vk* const* vks, const swb_fr* const* public_inputs, const size_t* n_inputs,
+                            const uint8_t* const* proofs, const size_t* lens, swb_rng* rng, int* ok) {
+    if (!c) return SWB_EARG;
+    if (n == 0) return SWB_OK;
+    SWB_REQUIRE(c, ok != nullptr, "verify_batch: ok is NULL");
+    for (size_t i = 0; i < n; i++) ok[i] = 0;
+    SWB_REQUIRE(c, vks && public_inputs && n_inputs && proofs && lens, "verify_batch: NULL argument");
+    std::vector<const VerifyingKey*> keys(n);
+    for (size_t i = 0; i < n; i++) {
+        SWB_REQUIRE(c, vks[i] && proofs[i] && (public_inputs[i] || !n_inputs[i]), "verify_batch: NULL key, proof or public inputs");
+        keys[i] = &vks[i]->h->vk;
+    }
+    ChaChaRng local;
+    if (!rng) {
+        uint8_t seed[32];
+        if (!os_entropy(seed)) return swb::set_err(c, SWB_EINTERNAL, "%s", "verify_batch: no rng given and no OS entropy source available");
+        local = ChaChaRng(seed, 12);
+    }
+    int rc;
+    try {
+        rc = marlin_verify_batch(c, n, keys.data(), reinterpret_cast<const uint64_t* const*>(public_inputs), n_inputs, proofs, lens,
+                                 rng ? rng->h.rng : local, ok);
+    } catch (const std::exception& e) {
+        rc = swb::set_err(c, SWB_EINTERNAL, "verify_batch: %s", e.what());
+    }
+    if (rc != SWB_OK)
+        for (size_t i = 0; i < n; i++) ok[i] = 0;
+    return rc;
 }
 void swb_bytes_free(uint8_t* p) { free(p); }
 

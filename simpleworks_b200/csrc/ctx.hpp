@@ -11,6 +11,12 @@
 #include "../../include/swb200.h"
 #include "fp.cuh"
 
+namespace swb {
+// A bucket shard: the MSM fills only the buckets b with b mod world == rank of every bucket set and returns that share of
+// the result (world a power of two; world = 1: all buckets)
+struct BucketShard { int rank, world; };
+}  // namespace swb
+
 struct swb_ctx {
     int device = 0;
     int sm_count = 0;
@@ -43,9 +49,10 @@ struct swb_ctx {
     size_t pinned_bytes = 0;
     uint32_t* pair_count_host = nullptr;   // pinned word: summed slots of the last pair-sum pass (profiling)
 
-    // MSM slots: slot 0 runs on `stream`; slots 1..MSM_SLOTS-1 have streams of their own (a normal one
-    // for sort + accumulation, a high-priority one for the latency-bound bucket tail) and their own
-    // scratch, so that independent MSMs of one prover round overlap (msm.cu: msm_begin / msm_end)
+    // MSM slots: slot 0 runs on `stream` (the swb_msm_* single calls and the queue's batches); slots 1..MSM_SLOTS-1
+    // have streams of their own (a normal one for sort + accumulation, a high-priority one for the latency-bound
+    // bucket tail) and their own scratch, so that the queue's independent MSMs overlap.  Only msm.cu starts and
+    // finishes MSMs on them.
     static constexpr int MSM_SLOTS = 3;
     struct MsmSlot {
         cudaStream_t work = nullptr, tail = nullptr;
@@ -58,6 +65,16 @@ struct swb_ctx {
         bool active = false, empty = false;
     } msm_slot[MSM_SLOTS];
     int scratch_slot = 0;              // suffix of scratch tags while a slot > 0 is being launched
+    // the MSM queue (msm_queue_* below): requests by id, from submission until their result is taken
+    struct MsmRequest {
+        const swb_bases* bases; size_t offset, n; const void* scalars; int montgomery; swb::BucketShard shard;
+        int slot = -1;                 // -1: noted; else the slot it was launched on
+        bool done = false;             // finished: the result is in `out`
+        swb_g1_jacobian out;
+    };
+    std::map<size_t, MsmRequest> msm_queue;
+    size_t msm_queue_next = 0;         // id of the next request
+    int msm_next_slot = 1;             // slot of the next single MSM (1 and 2 alternately)
     // bucket sharding of the swb_msm_* entry points (swb_msm_set_bucket_shard, swb::BucketShard)
     int bucket_rank = 0, bucket_world = 1;
     // multi-GPU proving (swb_set_msm_shard): this rank's share of every prover MSM, and who adds them up
@@ -92,21 +109,20 @@ int set_err(swb_ctx* c, int code, const char* fmt, ...);
 // wait for the context's stream and for the MSM slots' own streams (before device memory they may be
 // reading is released)
 void sync_all_streams(swb_ctx* c);
-// A bucket shard: the MSM fills only the buckets b with b mod world == rank of every bucket set and returns that share of
-// the result (world a power of two; world = 1: all buckets)
-struct BucketShard { int rank, world; };
-// One MSM split in two: msm_begin enqueues everything up to the device->host copy of the bucket-set
-// sums (slot 0: on the context's stream; slot > 0: on the slot's own streams, after the work already
-// queued on the context's stream), msm_end waits for it and finishes on the host.  A slot holds one
-// MSM at a time.
-int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
-              BucketShard shard);
-// Several scalar vectors over one handle WITH window tables as ONE MSM pipeline (one sort, one accumulation, one bucket
-// reduction; a bucket set per vector): msm_end then delivers `count` results.  msm_can_batch says whether a list qualifies.
-bool msm_can_batch(swb_ctx* c, const swb_bases* bases, size_t count, const size_t* ns);
-int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, const size_t* offsets, const void* const* scalars_dev,
-                    const size_t* ns, int montgomery, BucketShard shard);
-int msm_end(swb_ctx* c, int slot, swb_g1_jacobian* out);
+// The MSM queue: submission checks a request and only notes it (its scalars must stay alive until the result is taken
+// or the queue abandoned).  A flush launches the noted requests: consecutive ones over the same bases, bucket shard and
+// scalar form make runs of up to MSM_MAX_BATCH; a run of two or more over window tables goes out as ONE batched pipeline,
+// every other request goes to slots 1 and 2 alternately, so that the bucket tail of one runs under the accumulation of
+// the next.  A result is the affine value as a Z = 1 Jacobian (Z = 0, and n = 0: the identity).
+int msm_queue_submit(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
+                     BucketShard shard, size_t* id);
+int msm_queue_flush(swb_ctx* c);
+// flushes when the request is still noted, waits for it and hands its result over (once)
+int msm_queue_result(swb_ctx* c, size_t id, swb_g1_jacobian* out);
+// launches and finishes every request, keeping the results (before the bases they read are replaced)
+int msm_queue_drain(swb_ctx* c);
+// waits for the launched requests, frees their slots and forgets every request (failure paths)
+void msm_queue_abandon(swb_ctx* c);
 // fixed_base.cu: the window-table width that suits MSMs of about n scalars (what swb_bases_precompute picks for
 // window_bits = 0)
 int tables_pick_window(size_t n);

@@ -6,6 +6,7 @@
 #pragma once
 #include <vector>
 
+#include "../../../include/swb200.h"
 #include "../g1_decode.cuh"
 #include "rng.hpp"
 
@@ -46,6 +47,18 @@ inline G1Point to_affine(const G1Xyzz& p) {
     r.y = p.y * (p.zz * inv);
     r.infinity = false;
     return r;
+}
+// an MSM result of the library: the affine value as a Z = 1 Jacobian, Z = 0 for the identity
+inline G1Point from_jacobian(const swb_g1_jacobian& o) {
+    G1Point p = G1Point::identity();
+    Fq z;
+    memcpy(z.l, o.z.l, 48);
+    if (!z.is_zero()) {
+        p.infinity = false;
+        memcpy(p.x.l, o.x.l, 48);
+        memcpy(p.y.l, o.y.l, 48);
+    }
+    return p;
 }
 inline G1Point g1_generator() {
     const uint32_t gx[12] = SWB_FQ_G1_GEN_X_INIT, gy[12] = SWB_FQ_G1_GEN_Y_INIT;

@@ -414,36 +414,15 @@ struct GpuEngine {
             if (c->trace) fprintf(stderr, "[swb trace] SRS window tables not built: %s\n", swb_last_error(c));
         }
     }
-    // Independent MSMs (the commitments of a round, the parts of an opening) are submitted first and
-    // collected later: two of them are in flight on the library's MSM slots, so the latency-bound
-    // bucket tail of one runs under the accumulation of the next.  The scalars must stay alive until the
-    // result has been collected.
-    // An MSM is first only NOTED (its scalars must stay alive until the result has been collected); the list is
-    // launched when a result is asked for: over window tables as ONE batched pipeline (msm_begin_batch: one sort, one
-    // accumulation, one bucket reduction for all commitments of a prover round), otherwise one after the other on the
-    // library's two MSM slots, whose bucket tails overlap with the next accumulation.
+    // The MSMs of a round (the commitments, the parts of an opening) go to the context's MSM queue (ctx.hpp:
+    // msm_queue_*), which batches them over window tables or overlaps them on its slots.  What the engine adds is the
+    // sharding over ranks: each rank submits its share of every MSM, and the shares are summed when a result is asked
+    // for.  The scalars must stay alive until the result has been taken.
     struct Ticket {
-        void* h; size_t offset; const Fr* scalars; size_t n;     // the request
-        bool launched, done, sharded, combined, by_bucket;
-        int slot;
-        G1Point value;
-        swb_g1_jacobian share;
+        bool sharded, combined;
+        G1Point value;                     // the sum over the ranks, once combined
     };
-    std::vector<Ticket> tickets;                           // ids ticket_base .. ; finished old ones are dropped in blocks
-    size_t ticket_base = 0;
-    long slot_owner[swb_ctx::MSM_SLOTS] = {-1, -1, -1};    // ticket id occupying each slot
-    int next_slot = 1;
-    static G1Point from_jacobian(const swb_g1_jacobian& out) {
-        G1Point p = G1Point::identity();
-        Fq z;
-        memcpy(z.l, out.z.l, 48);
-        if (!z.is_zero()) {                 // the library returns Z = 1
-            p.infinity = false;
-            memcpy(p.x.l, out.x.l, 48);
-            memcpy(p.y.l, out.y.l, 48);
-        }
-        return p;
-    }
+    std::map<size_t, Ticket> tickets;      // by queue id; erased when msm_result hands the value over
     bool sharding() const { return c->shard_world > 1 && (c->shard_combine || c->comm); }
     // Power-of-two worlds shard by BUCKET (swb::BucketShard: every rank sees the whole polynomial -- it
     // has it anyway -- and fills its interleaved share of the buckets, so accumulation AND bucket reduction shrink
@@ -452,149 +431,66 @@ struct GpuEngine {
     // (only over bases with window tables: on the plain path every rank would still sort all pairs, and the index
     // split measured slightly faster -- 2^20 constraints on two GPUs: 0.248 s against 0.256 s)
     bool bucket_mode(const swb_bases* b) const { return shards_by_bucket() && b && b->tab_w > 0; }
-    // the bucket shard ticket t runs under: this rank's share for a by-bucket ticket, else the context's own
-    BucketShard bucket_shard(const Ticket& t) const {
-        return t.by_bucket ? BucketShard{c->shard_rank, c->shard_world} : BucketShard{c->bucket_rank, c->bucket_world};
+    // the bucket shard an MSM runs under: this rank's share when it shards by bucket, else the context's own
+    BucketShard bucket_shard(bool by_bucket) const {
+        return by_bucket ? BucketShard{c->shard_rank, c->shard_world} : BucketShard{c->bucket_rank, c->bucket_world};
     }
-    void finish(Ticket& t) {
-        t.done = true;
-        if (!t.sharded) {
-            t.value = from_jacobian(t.share);
-            t.combined = true;
-        }
-    }
-    // this rank's part of ticket t as (offset, scalars, n)
-    void local_part(const Ticket& t, size_t* off, const Fr** sc, size_t* n) const {
-        *off = t.offset; *sc = t.scalars; *n = t.n;
-        if (t.sharded && !t.by_bucket) {       // contiguous share of the index range (remainder to the first ranks)
-            const size_t base = t.n / (size_t)c->shard_world, rem = t.n % (size_t)c->shard_world, r = (size_t)c->shard_rank;
-            const size_t lo = r * base + (r < rem ? r : rem);
-            *off = t.offset + lo; *sc = t.scalars + lo; *n = base + (r < rem ? 1 : 0);
-        }
-    }
-    void launch_single(size_t id) {
-        Ticket& t = tickets.at(id - ticket_base);
-        const int slot = next_slot;
-        next_slot = next_slot == 1 ? 2 : 1;
-        if (slot_owner[slot] >= 0) collect((size_t)slot_owner[slot]);
-        size_t off, n;
-        const Fr* sc;
-        local_part(t, &off, &sc, &n);
-        ck(msm_begin(c, slot, static_cast<swb_bases*>(t.h), off, sc, n, 1, bucket_shard(t)), "msm");
-        t.launched = true;
-        t.slot = slot;
-        slot_owner[slot] = (long)id;
-    }
-    // launches every noted ticket; runs of tickets over the same table-backed handle go out as batches
-    void flush() {
-        size_t k = 0;
-        while (k < tickets.size()) {
-            if (tickets[k].launched) { k++; continue; }
-            size_t e = k;
-            std::vector<size_t> offs, ns;
-            std::vector<const void*> scs;
-            while (e < tickets.size() && !tickets[e].launched && tickets[e].h == tickets[k].h &&
-                   tickets[e].sharded == tickets[k].sharded && tickets[e].by_bucket == tickets[k].by_bucket && e - k < (size_t)MSM_MAX_BATCH) {
-                size_t off, n;
-                const Fr* sc;
-                local_part(tickets[e], &off, &sc, &n);
-                offs.push_back(off); ns.push_back(n); scs.push_back(sc);
-                e++;
-            }
-            swb_bases* b = static_cast<swb_bases*>(tickets[k].h);
-            if (e - k >= 2 && msm_can_batch(c, b, e - k, ns.data())) {
-                // the slots must be idle: the batch runs on the context's stream with slot 0's scratch
-                for (int sl = 1; sl < swb_ctx::MSM_SLOTS; sl++)
-                    if (slot_owner[sl] >= 0) collect((size_t)slot_owner[sl]);
-                ck(msm_begin_batch(c, 0, b, e - k, offs.data(), scs.data(), ns.data(), 1, bucket_shard(tickets[k])), "msm (batch)");
-                std::vector<swb_g1_jacobian> outs(e - k);
-                ck(msm_end(c, 0, outs.data()), "msm (batch)");
-                for (size_t q = k; q < e; q++) {
-                    tickets[q].launched = true;
-                    tickets[q].slot = 0;
-                    tickets[q].share = outs[q - k];
-                    finish(tickets[q]);
-                }
-            } else {
-                for (size_t q = k; q < e; q++) launch_single(ticket_base + q);
-            }
-            k = e;
-        }
-    }
-    // finishes the local part of a ticket (this rank's share when sharded)
-    void collect(size_t id) {
-        Ticket& t = tickets.at(id - ticket_base);
-        if (t.done) return;
-        if (!t.launched) flush();
-        if (t.done) return;
-        ck(msm_end(c, t.slot, &t.share), "msm");
-        slot_owner[t.slot] = -1;
-        finish(t);
+    // this rank's part [lo, lo + count) of an MSM of n scalars sharded by index (remainder to the first ranks): the count
+    size_t local_part(size_t n, size_t* lo) const {
+        const size_t base = n / (size_t)c->shard_world, rem = n % (size_t)c->shard_world, r = (size_t)c->shard_rank;
+        *lo = r * base + (r < rem ? r : rem);
+        return base + (r < rem ? 1 : 0);
     }
     // shares -> sums over all ranks.  With the library's communicator every share that is outstanding (the
     // commitments of a round are all submitted before the first result is asked for) goes into ONE all-gather;
     // a caller-supplied callback is invoked per MSM.
     void combine_pending() {
         std::vector<size_t> ids;
-        for (size_t k = 0; k < tickets.size(); k++)
-            if (tickets[k].sharded && !tickets[k].combined) ids.push_back(ticket_base + k);
-        if (ids.empty()) return;
-        for (size_t id : ids) collect(id);
-        if (c->shard_combine) {
-            for (size_t id : ids) {
-                Ticket& t = tickets.at(id - ticket_base);
-                swb_g1_jacobian sum;
-                if (c->shard_combine(c->shard_user, &t.share, &sum) != 0) throw MarlinError("msm: combining the ranks' partial results failed");
-                t.value = from_jacobian(sum);
-                t.combined = true;
-            }
-            return;
-        }
+        for (auto& kv : tickets)
+            if (kv.second.sharded && !kv.second.combined) ids.push_back(kv.first);
         std::vector<swb_g1_jacobian> mine(ids.size()), sums(ids.size());
-        for (size_t k = 0; k < ids.size(); k++) mine[k] = tickets.at(ids[k] - ticket_base).share;
-        ck(comm_sum_g1(c, mine.data(), mine.size(), sums.data()), "msm (all-gather of the partial results)");
-        for (size_t k = 0; k < ids.size(); k++) {
-            Ticket& t = tickets.at(ids[k] - ticket_base);
-            t.value = from_jacobian(sums[k]);
-            t.combined = true;
+        for (size_t k = 0; k < ids.size(); k++) ck(msm_queue_result(c, ids[k], &mine[k]), "msm");
+        if (c->shard_combine) {
+            for (size_t k = 0; k < ids.size(); k++)
+                if (c->shard_combine(c->shard_user, &mine[k], &sums[k]) != 0) throw MarlinError("msm: combining the ranks' partial results failed");
+        } else {
+            ck(comm_sum_g1(c, mine.data(), mine.size(), sums.data()), "msm (all-gather of the partial results)");
         }
+        for (size_t k = 0; k < ids.size(); k++) tickets.at(ids[k]) = Ticket{true, true, from_jacobian(sums[k])};
     }
     // (sizes the SRS window tables: in a power-of-two world they will be used by bucket, i.e. on whole polynomials)
     size_t msm_local_count(size_t n) {
-        if (!sharding() || shards_by_bucket()) return n;
-        const size_t base = n / (size_t)c->shard_world, rem = n % (size_t)c->shard_world;
-        return base + ((size_t)c->shard_rank < rem ? 1 : 0);
+        size_t lo;
+        return !sharding() || shards_by_bucket() ? n : local_part(n, &lo);
     }
     size_t msm_submit(void* h, size_t offset, const Vec& scalars, size_t n) {
         OpTimer ot_(c, "msm_submit");
-        if (tickets.size() >= 128) {                       // batches are a handful of MSMs: these are long finished
-            for (size_t i = 0; i < 64; i++) collect(ticket_base + i);
-            combine_pending();
-            tickets.erase(tickets.begin(), tickets.begin() + 64);
-            ticket_base += 64;
-        }
-        Ticket t{};
-        t.h = h; t.offset = offset; t.scalars = scalars.p; t.n = n;
-        t.sharded = sharding();
-        t.by_bucket = bucket_mode(static_cast<swb_bases*>(h));
-        t.slot = -1;
-        t.value = G1Point::identity();
-        tickets.push_back(t);
-        return ticket_base + tickets.size() - 1;
+        const swb_bases* b = static_cast<swb_bases*>(h);
+        const bool sharded = sharding(), by_bucket = bucket_mode(b);
+        size_t lo = 0, id = 0;
+        if (sharded && !by_bucket) n = local_part(n, &lo);
+        ck(msm_queue_submit(c, b, offset + lo, scalars.p + lo, n, 1, bucket_shard(by_bucket), &id), "msm");
+        tickets[id] = Ticket{sharded, false, G1Point::identity()};
+        return id;
     }
     G1Point msm_result(size_t id) {
         OpTimer ot_(c, "msm_result");
-        collect(id);
-        if (!tickets.at(id - ticket_base).combined) combine_pending();
-        return tickets.at(id - ticket_base).value;
+        Ticket& t = tickets.at(id);
+        if (!t.sharded) {
+            swb_g1_jacobian out;
+            ck(msm_queue_result(c, id, &out), "msm");
+            t.value = from_jacobian(out);
+        } else if (!t.combined) {
+            combine_pending();
+        }
+        const G1Point v = t.value;
+        tickets.erase(id);
+        return v;
     }
-    void msm_drain() {
-        for (size_t i = 0; i < tickets.size(); i++) collect(ticket_base + i);
-        combine_pending();
-    }
-    ~GpuEngine() {
-        try { msm_drain(); } catch (...) {}
-    }
+    // the tables replace the bases: every MSM must have finished (the results stay in the queue)
+    void msm_drain() { ck(msm_queue_drain(c), "msm"); }
+    // after a failed call: the MSMs of the call are forgotten, their scalars are gone
+    void msm_abandon() { tickets.clear(); msm_queue_abandon(c); }
 };
 using Api = MarlinApi<GpuEngine>;
 
@@ -705,6 +601,7 @@ int swb_marlin_index(swb_ctx* c, const swb_srs* srs, const swb_r1cs* cs, swb_pk*
     GpuEngine eng(c);
     int rc = Api::index(eng, srs->h, cs->h, &p->h, &v->h, &err);
     if (rc) {
+        srs->h->srs->eng->msm_abandon();
         delete p;
         delete v;
         return swb::set_err(c, SWB_EINTERNAL, "index: %s", err.c_str());
@@ -732,7 +629,10 @@ int swb_marlin_prove(swb_ctx* c, const swb_pk* pk, const swb_r1cs* cs, swb_rng* 
     std::string err;
     GpuEngine eng(c);
     int rc = Api::prove(eng, pk->h, cs->h, &rng->h, proof, len, &err);
-    if (rc) return swb::set_err(c, SWB_EINTERNAL, "prove: %s", err.c_str());
+    if (rc) {
+        pk->h->pk.ck.srs->eng->msm_abandon();
+        return swb::set_err(c, SWB_EINTERNAL, "prove: %s", err.c_str());
+    }
     return SWB_OK;
 }
 int swb_marlin_verify(swb_ctx* c, const swb_vk* vk, const swb_fr* public_inputs, size_t n, const uint8_t* proof, size_t len,
@@ -766,6 +666,7 @@ int swb_marlin_verify_batch(swb_ctx* c, size_t n, const swb_vk* const* vks, cons
         rc = marlin_verify_batch(c, n, keys.data(), reinterpret_cast<const uint64_t* const*>(public_inputs), n_inputs, proofs, lens,
                                  rng ? rng->h.rng : local, ok);
     } catch (const std::exception& e) {
+        msm_queue_abandon(c);
         rc = swb::set_err(c, SWB_EINTERNAL, "verify_batch: %s", e.what());
     }
     if (rc != SWB_OK)
@@ -969,6 +870,7 @@ int swb_pk_deserialize(swb_ctx* c, const uint8_t* bytes, size_t len, swb_pk** pk
         else swb_vk_free(v);
         return SWB_OK;
     } catch (const std::exception& e) {
+        if (s) s->eng.msm_abandon();
         if (p) { delete p->h; delete p; }
         if (v) swb_vk_free(v);
         if (s) srs_release(s);

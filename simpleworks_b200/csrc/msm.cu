@@ -23,8 +23,8 @@
 //
 // With window tables (swb_bases_precompute, fixed_base.cu) digit j of a scalar selects the precomputed
 // point 2^(c*j) * P, so all digits share ONE bucket set: steps 2-6 run on a single segment of n * W
-// pairs and step 7 has nothing to fold.  msm_begin / msm_end split a call so that independent MSMs
-// overlap on slots with streams and scratch of their own.
+// pairs and step 7 has nothing to fold.  msm_begin / msm_end split a call so that the independent MSMs of the
+// queue (msm_queue_*, ctx.hpp) overlap on slots with streams and scratch of their own.
 //
 // The result is the affine value (as a Z = 1 Jacobian), which is unique, hence bit-identical to
 // what arkworks' callers see after into_affine().
@@ -95,7 +95,7 @@ static bool msm_use_tables(const swb_ctx* c, const swb_bases* b, size_t n, size_
 }
 
 // can these vectors run as ONE batched MSM (one bucket set each over the handle's window tables)?
-bool msm_can_batch(swb_ctx* c, const swb_bases* bases, size_t count, const size_t* ns) {
+static bool msm_can_batch(swb_ctx* c, const swb_bases* bases, size_t count, const size_t* ns) {
     if (!bases || count < 2 || count > (size_t)MSM_MAX_BATCH) return false;
     size_t total = 0;
     for (size_t k = 0; k < count; k++) total += ns[k];
@@ -159,18 +159,30 @@ static int msm_plan(swb_ctx* c, const swb_bases* bases, const MsmBatch& batch, B
     return SWB_OK;
 }
 
-int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, const size_t* offsets, const void* const* scalars_dev,
-                    const size_t* ns, int montgomery, BucketShard shard) {
+// the checks of one request, made by the single calls and at submission to the queue
+static int msm_check(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n) {
+    SWB_REQUIRE(c, bases != nullptr, "msm: bad batch");
+    SWB_REQUIRE(c, bases->ctx == c, "msm: bases belong to another context");
+    SWB_REQUIRE(c, offset <= bases->n && n <= bases->n - offset, "msm: offset + n exceeds the loaded bases");
+    SWB_REQUIRE(c, n == 0 || scalars_dev != nullptr, "msm: NULL scalars");
+    SWB_REQUIRE(c, n < ((size_t)1 << 31), "msm: n must be < 2^31");
+    return SWB_OK;
+}
+
+// One MSM split in two: msm_begin enqueues everything up to the device->host copy of the bucket-set sums (slot 0: on the
+// context's stream; slot > 0: on the slot's own streams, after the work already queued on the context's stream), msm_end
+// waits for it and finishes on the host.  A slot holds one MSM at a time.  msm_begin_batch runs several scalar vectors
+// over one handle with window tables as ONE pipeline (a bucket set per vector, see msm_can_batch); msm_end then
+// delivers `count` results.  Every vector has passed msm_check.
+static int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, const size_t* offsets, const void* const* scalars_dev,
+                           const size_t* ns, int montgomery, BucketShard shard) {
     SWB_REQUIRE(c, slot >= 0 && slot < swb_ctx::MSM_SLOTS, "msm: bad slot");
     SWB_REQUIRE(c, !c->msm_slot[slot].active, "msm: slot already holds an MSM");
-    SWB_REQUIRE(c, bases != nullptr && count >= 1 && count <= (size_t)MSM_MAX_BATCH && offsets && scalars_dev && ns, "msm: bad batch");
-    SWB_REQUIRE(c, bases->ctx == c, "msm: bases belong to another context");
+    SWB_REQUIRE(c, count >= 1 && count <= (size_t)MSM_MAX_BATCH, "msm: bad batch");
     MsmBatch batch{};
     size_t total = 0;
     uint32_t kept = 0;
     for (size_t k = 0; k < count; k++) {
-        SWB_REQUIRE(c, offsets[k] <= bases->n && ns[k] <= bases->n - offsets[k], "msm: offset + n exceeds the loaded bases");
-        SWB_REQUIRE(c, ns[k] == 0 || scalars_dev[k] != nullptr, "msm: NULL scalars");
         // empty vectors keep their bucket set (it stays empty), so that results stay in the caller's order
         batch.scalars[kept] = (const uint32_t*)scalars_dev[k];
         batch.start[kept] = (uint32_t)total;
@@ -208,13 +220,13 @@ int msm_begin_batch(swb_ctx* c, int slot, const swb_bases* bases, size_t count, 
     return rc;
 }
 
-int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
-              BucketShard shard) {
+static int msm_begin(swb_ctx* c, int slot, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
+                     BucketShard shard) {
     return msm_begin_batch(c, slot, bases, 1, &offset, &scalars_dev, &n, montgomery, shard);
 }
 
 // outs: one result per vector of the batch (one for a plain msm_begin)
-int msm_end(swb_ctx* c, int slot, swb_g1_jacobian* out) {
+static int msm_end(swb_ctx* c, int slot, swb_g1_jacobian* out) {
     SWB_REQUIRE(c, slot >= 0 && slot < swb_ctx::MSM_SLOTS && out, "msm: bad slot");
     swb_ctx::MsmSlot& sl = c->msm_slot[slot];
     SWB_REQUIRE(c, sl.active, "msm: slot holds no MSM");
@@ -267,7 +279,8 @@ static BucketShard ctx_bucket_shard(const swb_ctx* c) { return {c->bucket_rank, 
 static int msm_run(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
                    swb_g1_jacobian* out) {
     SWB_REQUIRE(c, out != nullptr, "msm: NULL argument");
-    int rc = msm_begin(c, 0, bases, offset, scalars_dev, n, montgomery, ctx_bucket_shard(c));
+    int rc = msm_check(c, bases, offset, scalars_dev, n);
+    if (rc == SWB_OK) rc = msm_begin(c, 0, bases, offset, scalars_dev, n, montgomery, ctx_bucket_shard(c));
     if (rc != SWB_OK) return rc;
     return msm_end(c, 0, out);
 }
@@ -284,6 +297,95 @@ static int msm_run_host(swb_ctx* c, const swb_bases* bases, size_t offset, const
         SWB_CUDA(c, cudaMemcpyAsync(d, scalars_host, n * 32, cudaMemcpyHostToDevice, c->stream));
     }
     return msm_run(c, bases, offset, d, n, montgomery, out);
+}
+
+// ---- the MSM queue (ctx.hpp) ----------------------------------------------------------------------
+
+int msm_queue_submit(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
+                     BucketShard shard, size_t* id) {
+    const int rc = msm_check(c, bases, offset, scalars_dev, n);
+    if (rc != SWB_OK) return rc;
+    *id = c->msm_queue_next++;
+    c->msm_queue.emplace(*id, swb_ctx::MsmRequest{bases, offset, n, scalars_dev, montgomery, shard});
+    return SWB_OK;
+}
+
+// finishes the request running on slot s, if there is one
+static int msm_queue_collect(swb_ctx* c, int s) {
+    for (auto& kv : c->msm_queue) {
+        swb_ctx::MsmRequest& r = kv.second;
+        if (r.slot != s || r.done) continue;
+        const int rc = msm_end(c, s, &r.out);
+        r.done = rc == SWB_OK;
+        return rc;
+    }
+    return SWB_OK;
+}
+
+int msm_queue_flush(swb_ctx* c) {
+    auto it = c->msm_queue.begin();
+    while (it != c->msm_queue.end()) {
+        const swb_ctx::MsmRequest& first = it->second;
+        if (first.slot >= 0) { ++it; continue; }
+        swb_ctx::MsmRequest* run[MSM_MAX_BATCH];
+        size_t offs[MSM_MAX_BATCH], ns[MSM_MAX_BATCH];
+        const void* scs[MSM_MAX_BATCH];
+        size_t cnt = 0;
+        for (; it != c->msm_queue.end() && cnt < (size_t)MSM_MAX_BATCH; ++it, ++cnt) {
+            swb_ctx::MsmRequest& r = it->second;
+            if (r.slot >= 0 || r.bases != first.bases || r.montgomery != first.montgomery || r.shard.rank != first.shard.rank ||
+                r.shard.world != first.shard.world)
+                break;
+            run[cnt] = &r;
+            offs[cnt] = r.offset; ns[cnt] = r.n; scs[cnt] = r.scalars;
+        }
+        int rc = SWB_OK;
+        if (cnt >= 2 && msm_can_batch(c, first.bases, cnt, ns)) {
+            // the batch runs on the context's stream with slot 0's scratch: the other slots finish first
+            for (int s = 1; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
+            swb_g1_jacobian outs[MSM_MAX_BATCH];
+            if (rc == SWB_OK) rc = msm_begin_batch(c, 0, first.bases, cnt, offs, scs, ns, first.montgomery, first.shard);
+            if (rc == SWB_OK) rc = msm_end(c, 0, outs);
+            if (rc != SWB_OK) return rc;
+            for (size_t k = 0; k < cnt; k++) { run[k]->slot = 0; run[k]->done = true; run[k]->out = outs[k]; }
+            continue;
+        }
+        for (size_t k = 0; k < cnt; k++) {
+            const int s = c->msm_next_slot;
+            c->msm_next_slot = s == 1 ? 2 : 1;
+            rc = msm_queue_collect(c, s);
+            if (rc == SWB_OK) rc = msm_begin(c, s, run[k]->bases, run[k]->offset, run[k]->scalars, run[k]->n, run[k]->montgomery, run[k]->shard);
+            if (rc != SWB_OK) return rc;
+            run[k]->slot = s;
+        }
+    }
+    return SWB_OK;
+}
+
+int msm_queue_result(swb_ctx* c, size_t id, swb_g1_jacobian* out) {
+    auto it = c->msm_queue.find(id);
+    SWB_REQUIRE(c, out != nullptr && it != c->msm_queue.end(), "msm queue: no such request (its result was taken, or the queue abandoned)");
+    int rc = it->second.slot < 0 ? msm_queue_flush(c) : SWB_OK;
+    if (rc == SWB_OK && !it->second.done) rc = msm_queue_collect(c, it->second.slot);
+    if (rc != SWB_OK) return rc;
+    *out = it->second.out;
+    c->msm_queue.erase(it);
+    return SWB_OK;
+}
+
+int msm_queue_drain(swb_ctx* c) {
+    int rc = msm_queue_flush(c);
+    for (int s = 1; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
+    return rc;
+}
+
+void msm_queue_abandon(swb_ctx* c) {
+    const std::string err = c->err;         // the failure that led here stays the context's last error
+    swb_g1_jacobian dummy;
+    for (int s = 0; s < swb_ctx::MSM_SLOTS; s++)
+        if (c->msm_slot[s].active) msm_end(c, s, &dummy);       // waits for the slot's work
+    c->msm_queue.clear();
+    c->err = err;
 }
 
 static int msm_enqueue(swb_ctx* c, int slot, const swb_bases* bases, const MsmBatch& batch, BucketShard shard, int montgomery) {
@@ -502,35 +604,12 @@ int swb_msm_g1_batch_dev(swb_ctx* c, const swb_bases* b, const size_t* offsets, 
                          size_t n_msms, int montgomery, swb_g1_jacobian* outs) {
     if (!c) return SWB_EARG;
     SWB_REQUIRE(c, n_msms == 0 || (offsets && scalars_dev && ns && outs), "msm_batch: NULL argument");
+    std::vector<size_t> ids(n_msms);
     int rc = SWB_OK;
-    // over window tables: ONE pipeline for up to MSM_MAX_BATCH vectors at a time (a bucket set each)
-    size_t done = 0;
-    while (done < n_msms && rc == SWB_OK) {
-        size_t cnt = n_msms - done < (size_t)MSM_MAX_BATCH ? n_msms - done : (size_t)MSM_MAX_BATCH;
-        if (cnt < 2 || !msm_can_batch(c, b, cnt, ns + done)) break;
-        rc = msm_begin_batch(c, 0, b, cnt, offsets + done, scalars_dev + done, ns + done, montgomery, ctx_bucket_shard(c));
-        if (rc == SWB_OK) rc = msm_end(c, 0, outs + done);
-        done += cnt;
-    }
-    if (rc != SWB_OK || done == n_msms) return rc;
-    // otherwise two MSMs in flight on slots 1 and 2: the bucket tail of one runs under the accumulation of the next
-    size_t pending[swb_ctx::MSM_SLOTS] = {0, 0, 0};
-    bool busy[swb_ctx::MSM_SLOTS] = {false, false, false};
-    for (size_t i = done; i < n_msms && rc == SWB_OK; i++) {
-        const int slot = 1 + (int)(i & 1);
-        if (busy[slot]) {
-            rc = msm_end(c, slot, &outs[pending[slot]]);
-            busy[slot] = false;
-            if (rc != SWB_OK) break;
-        }
-        rc = msm_begin(c, slot, b, offsets[i], scalars_dev[i], ns[i], montgomery, ctx_bucket_shard(c));
-        if (rc == SWB_OK) { busy[slot] = true; pending[slot] = i; }
-    }
-    for (int slot = 1; slot < swb_ctx::MSM_SLOTS; slot++)
-        if (busy[slot]) {
-            const int r2 = msm_end(c, slot, &outs[pending[slot]]);    // always drain, keep the first error
-            if (rc == SWB_OK) rc = r2;
-        }
+    for (size_t i = 0; i < n_msms && rc == SWB_OK; i++)
+        rc = msm_queue_submit(c, b, offsets[i], scalars_dev[i], ns[i], montgomery, ctx_bucket_shard(c), &ids[i]);
+    for (size_t i = 0; i < n_msms && rc == SWB_OK; i++) rc = msm_queue_result(c, ids[i], &outs[i]);
+    if (rc != SWB_OK) msm_queue_abandon(c);
     return rc;
 }
 

@@ -52,7 +52,7 @@ struct BatchProof {
 };
 
 // the index of p among pts, or -1 (a point of the key)
-long slot_of(const std::vector<G1Point*>& pts, const G1Point* p) {
+long position_of(const std::vector<G1Point*>& pts, const G1Point* p) {
     for (size_t i = 0; i < pts.size(); i++)
         if (pts[i] == p) return (long)i;
     return -1;
@@ -62,18 +62,6 @@ void add_term(Terms& ts, const G1Point* p, const Fr& s) {
         if (t.first == p) { t.second = t.second + s; return; }
     ts.push_back({p, s});
 }
-G1Point from_result(const swb_g1_jacobian& o) {       // msm_end returns Z = 1, or Z = 0 for the identity
-    G1Point p = G1Point::identity();
-    Fq z;
-    memcpy(z.l, o.z.l, 48);
-    if (!z.is_zero()) {
-        p.infinity = false;
-        memcpy(p.x.l, o.x.l, 48);
-        memcpy(p.y.l, o.y.l, 48);
-    }
-    return p;
-}
-
 // runs body(j) for j < n on all cores; the first exception is rethrown afterwards
 template <class F>
 void parallel_for(size_t n, F&& body) {
@@ -184,7 +172,7 @@ int marlin_verify_batch(swb_ctx* c, size_t n, const VerifyingKey* const* vks, co
         if (!verify_prepare(*vks[j], pi, b.pr, rho[j], fold[j], &t)) { b.live = false; return; }
         for (int side = 0; side < 2; side++) {
             for (auto& term : side ? t.w : t.c) {
-                const long s = slot_of(b.pts, term.first);
+                const long s = position_of(b.pts, term.first);
                 if (s < 0) add_term(b.key_terms, term.first, term.second);      // only A has key points
                 else if (!term.first->infinity) {
                     Fr& dst = sc[side * total + base[k] + (size_t)s];
@@ -218,8 +206,10 @@ int marlin_verify_batch(swb_ctx* c, size_t n, const VerifyingKey* const* vks, co
             if (a >= e || live_before[e] == live_before[a]) continue;
             // the MSMs run over the whole bucket range whatever the context's bucket shard: a share would be useless here
             const BucketShard whole{0, 1};
-            const int r1 = msm_begin(c, 1, &bases, base[a], sc_dev + base[a], base[e] - base[a], 1, whole);
-            const int r2 = r1 == SWB_OK ? msm_begin(c, 2, &bases, base[a], sc_dev + total + base[a], base[e] - base[a], 1, whole) : r1;
+            size_t ida, idb;
+            fail(msm_queue_submit(c, &bases, base[a], sc_dev + base[a], base[e] - base[a], 1, whole, &ida), "verify_batch: msm");
+            fail(msm_queue_submit(c, &bases, base[a], sc_dev + total + base[a], base[e] - base[a], 1, whole, &idb), "verify_batch: msm");
+            fail(msm_queue_flush(c), "verify_batch: msm");
             Terms key;                                  // (on the host while the two MSMs run)
             for (size_t k = a; k < e; k++)
                 if (bp[order[k]].live)
@@ -228,11 +218,10 @@ int marlin_verify_batch(swb_ctx* c, size_t n, const VerifyingKey* const* vks, co
             for (auto& t : key) kv.push_back({*t.first, t.second});
             const G1Point key_part = to_affine(g1_msm_host(kv));
             swb_g1_jacobian ra, rb;
-            const int e1 = r1 == SWB_OK ? msm_end(c, 1, &ra) : r1;
-            const int e2 = r2 == SWB_OK ? msm_end(c, 2, &rb) : r2;
-            fail(e1 != SWB_OK ? e1 : e2, "verify_batch: msm");
-            pairs.push_back({g1_add(from_result(ra), key_part), group_key[g]->h});
-            pairs.push_back({g1_neg(from_result(rb)), group_key[g]->beta_h});
+            fail(msm_queue_result(c, ida, &ra), "verify_batch: msm");
+            fail(msm_queue_result(c, idb, &rb), "verify_batch: msm");
+            pairs.push_back({g1_add(from_jacobian(ra), key_part), group_key[g]->h});
+            pairs.push_back({g1_neg(from_jacobian(rb)), group_key[g]->beta_h});
         }
         return pairs;
     };

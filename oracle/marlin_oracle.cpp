@@ -32,7 +32,6 @@ struct CpuBases {
 };
 
 struct CpuEngine : HostVecOps {
-    static constexpr bool kDeviceIndex = false;     // index(): the host arithmetisation of marlin.hpp
     void vntt(Vec& v, uint32_t log_n, bool inverse, bool coset) {
         if (v.size() != ((size_t)1 << log_n)) throw MarlinError("vntt: size mismatch");
         orc_ntt(reinterpret_cast<fr_t*>(v.data()), log_n, inverse, coset, 0);
@@ -160,7 +159,7 @@ void orc_srs_free(void* srs) { delete static_cast<SrsHandle<CpuEngine>*>(srs); }
 int orc_marlin_index(void* srs, void* cs, void** pk, void** vk) {
     PkHandle<CpuEngine>* p = nullptr;
     VkHandle* v = nullptr;
-    int rc = Api::index(g_engine, static_cast<SrsHandle<CpuEngine>*>(srs), static_cast<R1csHandle*>(cs), &p, &v, &g_err);
+    int rc = Api::index(static_cast<SrsHandle<CpuEngine>*>(srs), static_cast<R1csHandle*>(cs), &p, &v, &g_err);
     *pk = p;
     *vk = v;
     return rc;
@@ -175,8 +174,8 @@ int orc_set_msm_shard(int rank, int world, int (*combine)(void*, const g1_jac_t*
     return 0;
 }
 int orc_marlin_prove(void* pk, void* cs, void* rng, uint8_t** bytes, size_t* len) {
-    return Api::prove(g_engine, static_cast<PkHandle<CpuEngine>*>(pk), static_cast<R1csHandle*>(cs), static_cast<RngHandle*>(rng),
-                      bytes, len, &g_err);
+    return Api::prove(static_cast<PkHandle<CpuEngine>*>(pk), static_cast<R1csHandle*>(cs), static_cast<RngHandle*>(rng), bytes, len,
+                      &g_err);
 }
 int orc_marlin_verify(void* vk, const uint64_t* pi, size_t n, const uint8_t* proof, size_t len, void* rng, int* ok) {
     return Api::verify(static_cast<VkHandle*>(vk), pi, n, proof, len, static_cast<RngHandle*>(rng), ok, &g_err);

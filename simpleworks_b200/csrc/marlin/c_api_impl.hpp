@@ -1,6 +1,7 @@
 // Engine-generic glue between the protocol templates (marlin.hpp) and a C ABI.  libswb200
 // instantiates it with the CUDA engine (marlin_abi.cu -> swb_marlin_*), the oracle build with the
-// CPU engine (oracle/marlin_oracle.cpp -> orc_marlin_*).
+// CPU engine (oracle/marlin_oracle.cpp -> orc_marlin_*).  setup binds an engine to the SRS it makes;
+// index and prove run on that SRS's engine.
 #pragma once
 #include <cstdio>
 #include <cstdlib>
@@ -164,25 +165,23 @@ struct MarlinApi {
             return 4;
         }
     }
-    static int index(Engine& eng, const SrsHandle<Engine>* srs, const R1csHandle* cs, PkHandle<Engine>** pk, VkHandle** vk,
-                     std::string* err) {
+    static int index(const SrsHandle<Engine>* srs, const R1csHandle* cs, PkHandle<Engine>** pk, VkHandle** vk, std::string* err) {
         try {
-            auto* p = new PkHandle<Engine>();
-            auto* v = new VkHandle();
-            marlin::index(eng, *srs->srs, cs->cs, &p->pk, &v->vk);
+            std::unique_ptr<PkHandle<Engine>> p(new PkHandle<Engine>());     // a key that fails mid-index is freed
+            std::unique_ptr<VkHandle> v(new VkHandle());
+            marlin::index(*srs->srs, cs->cs, &p->pk, &v->vk);
             host_profile().report("index");
-            *pk = p;
-            *vk = v;
+            *pk = p.release();
+            *vk = v.release();
             return 0;
         } catch (const std::exception& e) {
             *err = e.what();
             return 4;
         }
     }
-    static int prove(Engine& eng, const PkHandle<Engine>* pk, const R1csHandle* cs, RngHandle* rng, uint8_t** bytes, size_t* len,
-                     std::string* err) {
+    static int prove(const PkHandle<Engine>* pk, const R1csHandle* cs, RngHandle* rng, uint8_t** bytes, size_t* len, std::string* err) {
         try {
-            Proof pr = marlin::prove(eng, pk->pk, cs->cs, rng->rng);
+            Proof pr = marlin::prove(pk->pk, cs->cs, rng->rng);
             host_profile().report("prove");
             std::vector<uint8_t> b = pr.serialize();
             *bytes = (uint8_t*)malloc(b.size());

@@ -11,21 +11,28 @@
 //
 // Template parameter Engine supplies the operators and owns the polynomial storage: Engine::Vec is
 // a vector of Fr living where the engine computes (HBM for the CUDA engine of libswb200, RAM for
-// the CPU arm), so round polynomials stay resident between NTTs, element-wise passes and MSMs:
+// the CPU arm), so round polynomials stay resident between NTTs, element-wise passes and MSMs.  An SRS
+// holds the one engine that serves it (UniversalSrs::eng); index, prove and the proving key use that one.
+// What the templates call (semantics: marlin/vec_host.hpp):
 //   struct Engine {
-//     using Vec = ...;   vzeros vfrom vhost vclone vresize vlen vget vset vmul vadd vsub vadd_scaled
-//                        vscale vlin vadd_offset veval vdiv_vanishing vdiv_linear vbatch_inverse
-//                        vshift_down vdomain            (semantics: marlin/vec_host.hpp)
+//     using Vec = ...;   vzeros vfrom vwrite vclone vresize vlen vget vset vmul vadd vsub vadd_scaled vscale
+//                        vlin vadd_offset veval vdiv_vanishing vdiv_linear vbatch_inverse vshift_down vdomain
+//                        vrand vwitness_evals
 //     void  vntt(Vec& v, uint32_t log_n, bool inverse, bool coset);            // size 2^log_n, in place
+//     // sparse matrices in CSR form, as opaque handles
+//     void* csr_upload_filled(const std::vector<uint32_t>& start, Fill fill);  // fill(col, coef) writes the entries
+//     IndexOut index_arith(void* a, void* b, void* c, size_t ncons, size_t nvar, size_t ninst, const Domain& H);
+//     Vec   vspmv(const void* m, const Vec& x, size_t nout, const Fr* weights);
+//     void  csr_free(void* m);
 //     void* bases_from_powers(const G1Point& g, const Fr& beta, size_t n);     // resident beta^i * g
 //     void  export_bases(void* h, size_t offset, size_t n, G1Point* out);
 //     void  free_bases(void* h);
 //     void  bases_tune(void* h, size_t typical_n);   // optional restructuring for MSMs of about typical_n scalars
 //     size_t msm_submit(void* h, size_t offset, const Vec& scalars, size_t n);   // queue an MSM (scalars stay alive)
 //     G1Point msm_result(size_t id);  void msm_drain();
-//     // sum s_i * base[offset+i]; needed only by engines whose msm_submit is msm_submit_sync (vec_host.hpp)
-//     G1Point msm(void* h, size_t offset, const Vec& scalars_mont, size_t n);
+//     size_t msm_local_count(size_t n);   // how many of n scalars this engine processes (its share when sharded)
 //   };
+// The CUDA engine also has bases_load, csr_download and msm_abandon, which only marlin_abi.cu calls.
 //
 // Verification is the pairing check of kzg10::batch_check on the host (marlin/pairing.hpp): the two
 // opening equations are folded with a verifier-side random scalar into one pairing-product test
@@ -270,29 +277,22 @@ template <class Engine>
 struct ProvingKey {
     IndexInfo info;
     Domain dom_h, dom_k, dom_x;
-    // joint arithmetisation: entry k of K is (constraint r_k, variable c_k)
-    std::vector<uint32_t> ent_row, ent_col;         // r_k, position of c_k in H (reindexed)
     std::vector<LabeledPoly<Engine>> index_polys;   // row, col, a_val, b_val, c_val, row_col (resident)
     typename Engine::Vec row_evals, col_evals, val_a_evals, val_b_evals, val_c_evals;   // on K (resident)
-    // matrices regrouped by H position of the column (for t = sum_M eta_M M^T r_alpha): entries of
-    // position p are t_ent[t_start[p] .. t_start[p+1]): (constraint row, which matrix, coefficient)
-    std::vector<uint32_t> t_start, t_row;
-    std::vector<uint8_t> t_mat;
-    std::vector<Fr> t_coef;
     std::vector<Commitment> index_comms;
-    CommitterKey<Engine> ck;
-    // the same matrices where the engine keeps its vectors (device memory for the CUDA engine):
-    // A, B, C in CSR over z = (instance | witness), and the regrouped entries above (tagged by matrix)
-    Engine* eng = nullptr;
+    CommitterKey<Engine> ck;        // ck.srs->eng is the engine of every operation on the key; the SRS outlives the key
+    // the matrices where the engine keeps its vectors (device memory for the CUDA engine): A, B, C in CSR over
+    // z = (instance | witness), and the entries of all three regrouped by the H position of their column, tagged by
+    // matrix (for t = sum_M eta_M M^T r_alpha)
     void *m_a = nullptr, *m_b = nullptr, *m_c = nullptr, *m_t = nullptr;
     ProvingKey() {}
     ProvingKey(const ProvingKey&) = delete;
     ProvingKey& operator=(const ProvingKey&) = delete;
     ~ProvingKey() {
-        if (!eng) return;
+        if (!ck.srs) return;
         void* ms[4] = {m_a, m_b, m_c, m_t};
         for (void* m : ms)
-            if (m) eng->csr_free(m);
+            if (m) ck.srs->eng->csr_free(m);
     }
 };
 // IndexVerifierKey: index info + index commitments + MarlinKZG10's VerifierKey (g, gamma_g, h, beta_h,
@@ -416,7 +416,8 @@ std::unique_ptr<UniversalSrs<Engine>> universal_setup(Engine& eng, size_t num_co
 }
 
 template <class Engine>
-void index(Engine& eng, const UniversalSrs<Engine>& srs, const R1cs& cs, ProvingKey<Engine>* pk, VerifyingKey* vk) {
+void index(const UniversalSrs<Engine>& srs, const R1cs& cs, ProvingKey<Engine>* pk, VerifyingKey* vk) {
+    Engine& eng = *srs.eng;
     ScopedPhase ph_total("total");
     std::unique_ptr<ScopedPhase> ph(new ScopedPhase("i0_pad"));
     // pad_input_for_indexer_and_prover + make_matrices_square without copying the matrices: the instance
@@ -434,182 +435,38 @@ void index(Engine& eng, const UniversalSrs<Engine>& srs, const R1cs& cs, Proving
     pk->dom_h = Domain(ncons);
     pk->dom_x = Domain(ninst);
     const Domain& H = pk->dom_h;
-    typename Engine::Vec rowcol_v;
-    auto upload_rows = [&](const std::vector<SparseRow>& m) {
+    // The engine arithmetises where its vectors live (index_ops.cu on the CUDA engine): here the three matrices are
+    // only flattened into CSR arrays and staged there -- they are needed there anyway, for z_A, z_B, z_C.
+    ph.reset(); ph.reset(new ScopedPhase("i4_upload"));
+    pk->ck.srs = &srs;             // from here on the key frees its matrices through srs.eng, also when index throws
+    auto stage_rows = [&](const std::vector<SparseRow>& m) {
         std::vector<uint32_t> start(ncons + 1, 0);
         for (size_t r = 0; r < ncons; r++) start[r + 1] = start[r] + (uint32_t)row_of(m, r).e.size();
-        std::vector<uint32_t> col(start.back());
-        std::vector<Fr> coef(start.back());
+        return eng.csr_upload_filled(start, [&](uint32_t* col, Fr* coef) {
 #pragma omp parallel for schedule(static)
-        for (size_t r = 0; r < m.size(); r++) {
-            uint32_t at = start[r];
-            for (auto& e : m[r].e) { col[at] = col_of(e.second); coef[at] = e.first; at++; }
-        }
-        return eng.csr_upload(start, col, coef, nullptr);
-    };
-    if constexpr (Engine::kDeviceIndex) {
-        // The engine arithmetises where its vectors live (index_ops.cu on the CUDA engine): the host only flattens the
-        // three matrices into CSR arrays and uploads them -- they are needed there anyway, for z_A, z_B, z_C.
-        ph.reset(); ph.reset(new ScopedPhase("i4_upload"));
-        pk->eng = srs.eng;
-        auto stage_rows = [&](const std::vector<SparseRow>& m) {
-            std::vector<uint32_t> start(ncons + 1, 0);
-            for (size_t r = 0; r < ncons; r++) start[r + 1] = start[r] + (uint32_t)row_of(m, r).e.size();
-            return eng.csr_upload_filled(start, [&](uint32_t* col, Fr* coef) {
-#pragma omp parallel for schedule(static)
-                for (size_t r = 0; r < m.size(); r++) {
-                    uint32_t at = start[r];
-                    for (auto& e : m[r].e) { col[at] = col_of(e.second); coef[at] = e.first; at++; }
-                }
-            });
-        };
-        pk->m_a = stage_rows(cs.a);
-        pk->m_b = stage_rows(cs.b);
-        pk->m_c = stage_rows(cs.c);
-        ph.reset(); ph.reset(new ScopedPhase("i2_arith"));
-        auto out = eng.index_arith(pk->m_a, pk->m_b, pk->m_c, ncons, nvar, ninst, H);
-        const size_t nnz = out.nnz;
-        pk->info = IndexInfo{nvar, ncons, nnz, ninst};
-        pk->dom_k = Domain(nnz);
-        if (ahp_max_degree(pk->info.num_constraints, nvar, nnz) > srs.max_degree)
-            throw MarlinError("index: circuit exceeds the universal SRS bound");
-        pk->row_evals = std::move(out.row); pk->col_evals = std::move(out.col);
-        pk->val_a_evals = std::move(out.va); pk->val_b_evals = std::move(out.vb); pk->val_c_evals = std::move(out.vc);
-        rowcol_v = std::move(out.rowcol);
-        pk->m_t = out.m_t;
-    } else {
-    ph.reset(); ph.reset(new ScopedPhase("i1_merge_rows"));
-    // joint sparsity pattern, row by row, columns in increasing order; rows are independent, so
-    // they are merged in parallel: pass 1 counts the distinct columns of each row, pass 2 fills
-    struct Ent { uint32_t col; uint8_t which; Fr coef; };
-    const size_t nrows = ncons;
-    auto merged_row = [&](size_t r, std::vector<Ent>& tmp) {
-        tmp.clear();
-        const SparseRow* rows[3] = {&row_of(cs.a, r), &row_of(cs.b, r), &row_of(cs.c, r)};
-        for (uint8_t w = 0; w < 3; w++)
-            for (auto& e : rows[w]->e) tmp.push_back(Ent{col_of(e.second), w, e.first});
-        std::stable_sort(tmp.begin(), tmp.end(), [](const Ent& x, const Ent& y) { return x.col < y.col; });
-    };
-    std::vector<size_t> row_off(nrows + 1, 0);
-#pragma omp parallel
-    {
-        std::vector<Ent> tmp;
-#pragma omp for schedule(static)
-        for (size_t r = 0; r < nrows; r++) {
-            merged_row(r, tmp);
-            size_t distinct = 0;
-            for (size_t k = 0; k < tmp.size(); k++) distinct += (k == 0 || tmp[k].col != tmp[k - 1].col);
-            row_off[r + 1] = distinct;
-        }
-    }
-    for (size_t r = 0; r < nrows; r++) row_off[r + 1] += row_off[r];
-    const size_t nnz = row_off[nrows];
-    std::vector<uint32_t> er(nnz), ec(nnz);
-    std::vector<Fr> va(nnz, Fr::zero()), vb(nnz, Fr::zero()), vc(nnz, Fr::zero());
-#pragma omp parallel
-    {
-        std::vector<Ent> tmp;
-#pragma omp for schedule(static)
-        for (size_t r = 0; r < nrows; r++) {
-            merged_row(r, tmp);
-            size_t at = row_off[r];
-            for (size_t k = 0; k < tmp.size(); k++) {
-                if (k && tmp[k].col != tmp[k - 1].col) at++;
-                er[at] = (uint32_t)r;
-                ec[at] = tmp[k].col;
-                Fr& dst = tmp[k].which == 0 ? va[at] : tmp[k].which == 1 ? vb[at] : vc[at];
-                dst = dst + tmp[k].coef;
+            for (size_t r = 0; r < m.size(); r++) {
+                uint32_t at = start[r];
+                for (auto& e : m[r].e) { col[at] = col_of(e.second); coef[at] = e.first; at++; }
             }
-        }
-    }
+        });
+    };
+    pk->m_a = stage_rows(cs.a);
+    pk->m_b = stage_rows(cs.b);
+    pk->m_c = stage_rows(cs.c);
+    ph.reset(); ph.reset(new ScopedPhase("i2_arith"));
+    auto out = eng.index_arith(pk->m_a, pk->m_b, pk->m_c, ncons, nvar, ninst, H);
+    pk->m_t = out.m_t;
+    const size_t nnz = out.nnz;
     pk->info = IndexInfo{nvar, ncons, nnz, ninst};
     pk->dom_k = Domain(nnz);
-    const Domain& K = pk->dom_k;
     if (ahp_max_degree(pk->info.num_constraints, nvar, nnz) > srs.max_degree)
         throw MarlinError("index: circuit exceeds the universal SRS bound");
-    ph.reset(); ph.reset(new ScopedPhase("i2_arith"));
-    const std::vector<Fr> h_el = H.elements();
-    // For entry k = (r, c): row_k = H[pos(c)] (the variable side, summed against z), col_k = H[r]
-    // (the constraint side, paired with r(alpha, .)).  val_M(k) = M[r][c] / u_H(row_k, row_k) with
-    // u_H(x, x) = |H| x^(|H|-1) = |H| / x on H, so that
-    //    sum_j z(j) t(j) = sum_r r(alpha, H[r]) (M z)(r)   for   t(X) = sum_k val(k) u_H(X,row_k) u_H(alpha,col_k).
-    pk->ent_row.resize(nnz);
-    pk->ent_col.resize(nnz);
-    // six |K|-long evaluation vectors, filled in parallel (entries past nnz: row = col = H[0], val = 0);
-    // raw buffers, because std::vector would first value-initialise 0.8 GB on one core
-    std::unique_ptr<Fr[]> row(new Fr[K.n]), col(new Fr[K.n]), vala(new Fr[K.n]), valb(new Fr[K.n]), valc(new Fr[K.n]),
-        rowcol(new Fr[K.n]);
-#pragma omp parallel for schedule(static)
-    for (size_t k = 0; k < K.n; k++) {
-        if (k >= nnz) {
-            row[k] = h_el[0]; col[k] = h_el[0];
-            vala[k] = Fr::zero(); valb[k] = Fr::zero(); valc[k] = Fr::zero();
-        } else {
-            const size_t pos = H.reindex_by_subdomain(pk->dom_x, ec[k]);
-            pk->ent_row[k] = er[k];
-            pk->ent_col[k] = (uint32_t)pos;
-            row[k] = h_el[pos];
-            col[k] = h_el[er[k]];
-            const Fr scale = row[k] * H.size_inv;
-            vala[k] = va[k] * scale; valb[k] = vb[k] * scale; valc[k] = vc[k] * scale;
-        }
-        rowcol[k] = row[k] * col[k];
-    }
-    pk->row_evals = eng.vfrom_ptr(row.get(), K.n); pk->col_evals = eng.vfrom_ptr(col.get(), K.n);
-    pk->val_a_evals = eng.vfrom_ptr(vala.get(), K.n); pk->val_b_evals = eng.vfrom_ptr(valb.get(), K.n);
-    pk->val_c_evals = eng.vfrom_ptr(valc.get(), K.n);
-    ph.reset(); ph.reset(new ScopedPhase("i3_transpose"));
-    {
-        // counting sort of all matrix entries by the H position of their column; the order inside one
-        // position is irrelevant (the entries are summed in exact field arithmetic), so both passes run
-        // in parallel with atomic cursors
-        std::vector<uint32_t> pos_of(nvar), cnt(H.n + 1, 0);
-#pragma omp parallel for schedule(static)
-        for (size_t v = 0; v < nvar; v++) pos_of[v] = (uint32_t)H.reindex_by_subdomain(pk->dom_x, v);
-        const std::vector<SparseRow>* ms[3] = {&cs.a, &cs.b, &cs.c};
-        for (int m = 0; m < 3; m++) {
-            const std::vector<SparseRow>& mat = *ms[m];
-#pragma omp parallel for schedule(static)
-            for (size_t r = 0; r < mat.size(); r++)
-                for (auto& e : mat[r].e) {
-                    uint32_t& slot = cnt[pos_of[col_of(e.second)] + 1];
-#pragma omp atomic
-                    slot++;
-                }
-        }
-        for (size_t i = 0; i < H.n; i++) cnt[i + 1] += cnt[i];
-        pk->t_start = cnt;
-        const size_t tot = cnt[H.n];
-        pk->t_row.resize(tot); pk->t_mat.resize(tot); pk->t_coef.resize(tot);
-        std::vector<uint32_t> cur(cnt.begin(), cnt.end() - 1);
-        for (int m = 0; m < 3; m++) {
-            const std::vector<SparseRow>& mat = *ms[m];
-#pragma omp parallel for schedule(static)
-            for (size_t r = 0; r < mat.size(); r++)
-                for (auto& e : mat[r].e) {
-                    uint32_t at;
-                    uint32_t& slot = cur[pos_of[col_of(e.second)]];
-#pragma omp atomic capture
-                    at = slot++;
-                    pk->t_row[at] = (uint32_t)r; pk->t_mat[at] = (uint8_t)m; pk->t_coef[at] = e.first;
-                }
-        }
-    }
-    ph.reset(); ph.reset(new ScopedPhase("i4_upload"));
-    {
-        pk->eng = srs.eng;          // lives as long as the SRS, which the key references anyway (ck.srs)
-        pk->m_a = upload_rows(cs.a);
-        pk->m_b = upload_rows(cs.b);
-        pk->m_c = upload_rows(cs.c);
-        pk->m_t = eng.csr_upload(pk->t_start, pk->t_row, pk->t_coef, &pk->t_mat);
-    }
-    rowcol_v = eng.vfrom_ptr(rowcol.get(), pk->dom_k.n);
-    }
+    pk->row_evals = std::move(out.row); pk->col_evals = std::move(out.col);
+    pk->val_a_evals = std::move(out.va); pk->val_b_evals = std::move(out.vb); pk->val_c_evals = std::move(out.vc);
     ph.reset(); ph.reset(new ScopedPhase("i5_polys_commit"));
     const char* names[6] = {"row", "col", "a_val", "b_val", "c_val", "row_col"};
     const Domain& K = pk->dom_k;
-    const size_t nnz = pk->info.num_non_zero;
-    const typename Engine::Vec* evs[6] = {&pk->row_evals, &pk->col_evals, &pk->val_a_evals, &pk->val_b_evals, &pk->val_c_evals, &rowcol_v};
+    const typename Engine::Vec* evs[6] = {&pk->row_evals, &pk->col_evals, &pk->val_a_evals, &pk->val_b_evals, &pk->val_c_evals, &out.rowcol};
     pk->index_polys.clear();
     for (int i = 0; i < 6; i++) {
         LabeledPoly<Engine> lp;
@@ -618,7 +475,6 @@ void index(Engine& eng, const UniversalSrs<Engine>& srs, const R1cs& cs, Proving
         eng.vntt(lp.poly, K.log_n, true, false);
         pk->index_polys.push_back(std::move(lp));
     }
-    pk->ck.srs = &srs;
     pk->ck.supported_degree = ahp_max_degree(pk->info.num_constraints, nvar, nnz);
     std::vector<Randomness> unused;
     pk->index_comms.clear();
@@ -778,7 +634,8 @@ inline void build_lcs(const Domain& H, const Domain& K, const Challenges& ch, co
 // prove (AHPForR1CS prover rounds + MarlinKZG10 commit/open; SURVEY A.9)
 // ------------------------------------------------------------------------------------------------
 template <class Engine>
-Proof prove(Engine& eng, const ProvingKey<Engine>& pk, const R1cs& cs, ChaChaRng& zk_rng) {
+Proof prove(const ProvingKey<Engine>& pk, const R1cs& cs, ChaChaRng& zk_rng) {
+    Engine& eng = *pk.ck.srs->eng;
     if (!cs.has_assignment) throw MarlinError("prove: constraint system has no assignment");
     // the assignment after pad_input_for_indexer_and_prover + make_matrices_square (the matrices
     // themselves live in the proving key): instance padded with zeros to a power of two, dummy

@@ -1,8 +1,12 @@
 // Host implementation of the Engine vector interface used by the protocol templates
-// (marlin.hpp): Vec = std::vector<Fr> in RAM, every operation a parallel loop.  The CPU arm
-// (oracle build) derives its engine from this; the CUDA engine (marlin_abi.cu) implements the same
-// interface on device memory so that polynomials stay in HBM between NTTs and MSMs.
+// (marlin.hpp): Vec = std::vector<Fr> in RAM, every operation (the index arithmetisation included) a
+// parallel loop.  The CPU arm (oracle build) derives its engine from this; the CUDA engine
+// (marlin_abi.cu) implements the same interface on device memory so that polynomials stay in HBM
+// between NTTs and MSMs.
 #pragma once
+#include <algorithm>
+#include <memory>
+
 #include "poly.hpp"
 #include "rng.hpp"
 #include "curve_host.hpp"
@@ -14,9 +18,7 @@ struct HostVecOps {
     using Vec = std::vector<Fr>;
     Vec vzeros(size_t n) { return Vec(n, Fr::zero()); }
     Vec vfrom(const std::vector<Fr>& h) { return h; }
-    Vec vfrom_ptr(const Fr* p, size_t n) { return Vec(p, p + n); }
     void vwrite(Vec& v, size_t at, const Fr* p, size_t n) { std::copy(p, p + n, v.begin() + at); }   // v[at .. at+n) = p
-    std::vector<Fr> vhost(const Vec& v) { return v; }
     Vec vclone(const Vec& v) { return v; }
     void vresize(Vec& v, size_t n) { v.resize(n, Fr::zero()); }
     size_t vlen(const Vec& v) {
@@ -78,12 +80,125 @@ struct HostVecOps {
         std::vector<Fr> coef;
         std::vector<uint8_t> tag;
     };
-    void* csr_upload(const std::vector<uint32_t>& start, const std::vector<uint32_t>& col, const std::vector<Fr>& coef,
-                     const std::vector<uint8_t>* tag) {
-        HostCsr* m = new HostCsr();
-        m->start = start; m->col = col; m->coef = coef;
-        if (tag) m->tag = *tag;
-        return m;
+    // start [nrows + 1]; the column and coefficient arrays are written by `fill(col, coef)`
+    template <class Fill>
+    void* csr_upload_filled(const std::vector<uint32_t>& start, Fill&& fill) {
+        std::unique_ptr<HostCsr> m(new HostCsr());
+        m->start = start;
+        m->col.resize(start.back());
+        m->coef.resize(start.back());
+        fill(m->col.data(), m->coef.data());
+        return m.release();
+    }
+    // Marlin's index arithmetisation (the contract of the CUDA engine's, index_ops.cu) over A, B, C as staged by
+    // csr_upload_filled: ncons rows each, columns already shifted by the instance padding.  Returns the joint sparsity
+    // pattern's size nnz, the six evaluation vectors on K and the matrices regrouped by the H position of their column
+    // (tagged by matrix), for the prover's t.
+    struct IndexOut { size_t nnz = 0; Vec row, col, va, vb, vc, rowcol; void* m_t = nullptr; };
+    IndexOut index_arith(void* ha, void* hb, void* hc, size_t ncons, size_t nvar, size_t ninst, const Domain& H) {
+        const HostCsr* ms[3] = {static_cast<HostCsr*>(ha), static_cast<HostCsr*>(hb), static_cast<HostCsr*>(hc)};
+        const Domain X(ninst);
+        std::unique_ptr<ScopedPhase> ph(new ScopedPhase("i1_merge_rows"));
+        // joint sparsity pattern, row by row, columns in increasing order; rows are independent, so
+        // they are merged in parallel: pass 1 counts the distinct columns of each row, pass 2 fills
+        struct Ent { uint32_t col; uint8_t which; Fr coef; };
+        auto merged_row = [&](size_t r, std::vector<Ent>& tmp) {
+            tmp.clear();
+            for (uint8_t w = 0; w < 3; w++)
+                for (uint32_t e = ms[w]->start[r]; e < ms[w]->start[r + 1]; e++) tmp.push_back(Ent{ms[w]->col[e], w, ms[w]->coef[e]});
+            std::stable_sort(tmp.begin(), tmp.end(), [](const Ent& x, const Ent& y) { return x.col < y.col; });
+        };
+        std::vector<size_t> row_off(ncons + 1, 0);
+#pragma omp parallel
+        {
+            std::vector<Ent> tmp;
+#pragma omp for schedule(static)
+            for (size_t r = 0; r < ncons; r++) {
+                merged_row(r, tmp);
+                size_t distinct = 0;
+                for (size_t k = 0; k < tmp.size(); k++) distinct += (k == 0 || tmp[k].col != tmp[k - 1].col);
+                row_off[r + 1] = distinct;
+            }
+        }
+        for (size_t r = 0; r < ncons; r++) row_off[r + 1] += row_off[r];
+        const size_t nnz = row_off[ncons];
+        std::vector<uint32_t> er(nnz), ec(nnz);
+        std::vector<Fr> sa(nnz, Fr::zero()), sb(nnz, Fr::zero()), sc(nnz, Fr::zero());
+#pragma omp parallel
+        {
+            std::vector<Ent> tmp;
+#pragma omp for schedule(static)
+            for (size_t r = 0; r < ncons; r++) {
+                merged_row(r, tmp);
+                size_t at = row_off[r];
+                for (size_t k = 0; k < tmp.size(); k++) {
+                    if (k && tmp[k].col != tmp[k - 1].col) at++;
+                    er[at] = (uint32_t)r;
+                    ec[at] = tmp[k].col;
+                    Fr& dst = tmp[k].which == 0 ? sa[at] : tmp[k].which == 1 ? sb[at] : sc[at];
+                    dst = dst + tmp[k].coef;
+                }
+            }
+        }
+        ph.reset();
+        // For entry k = (r, c): row_k = H[pos(c)] (the variable side, summed against z), col_k = H[r]
+        // (the constraint side, paired with r(alpha, .)).  val_M(k) = M[r][c] / u_H(row_k, row_k) with
+        // u_H(x, x) = |H| x^(|H|-1) = |H| / x on H, so that
+        //    sum_j z(j) t(j) = sum_r r(alpha, H[r]) (M z)(r)   for   t(X) = sum_k val(k) u_H(X,row_k) u_H(alpha,col_k).
+        // Entries past nnz: row = col = H[0], val = 0.
+        const size_t kn = Domain(nnz).n;
+        const std::vector<Fr> h_el = H.elements();
+        IndexOut out;
+        out.nnz = nnz;
+        out.row = Vec(kn); out.col = Vec(kn); out.va = Vec(kn); out.vb = Vec(kn); out.vc = Vec(kn); out.rowcol = Vec(kn);
+#pragma omp parallel for schedule(static)
+        for (size_t k = 0; k < kn; k++) {
+            if (k >= nnz) {
+                out.row[k] = h_el[0]; out.col[k] = h_el[0];
+            } else {
+                out.row[k] = h_el[H.reindex_by_subdomain(X, ec[k])];
+                out.col[k] = h_el[er[k]];
+                const Fr scale = out.row[k] * H.size_inv;
+                out.va[k] = sa[k] * scale; out.vb[k] = sb[k] * scale; out.vc[k] = sc[k] * scale;
+            }
+            out.rowcol[k] = out.row[k] * out.col[k];
+        }
+        ph.reset(new ScopedPhase("i3_transpose"));
+        // counting sort of all matrix entries by the H position of their column; the order inside one
+        // position is irrelevant (the entries are summed in exact field arithmetic), so both passes run
+        // in parallel with atomic cursors
+        std::vector<uint32_t> pos_of(nvar), cnt(H.n + 1, 0);
+#pragma omp parallel for schedule(static)
+        for (size_t v = 0; v < nvar; v++) pos_of[v] = (uint32_t)H.reindex_by_subdomain(X, v);
+        for (int w = 0; w < 3; w++) {
+            const HostCsr& m = *ms[w];
+#pragma omp parallel for schedule(static)
+            for (size_t e = 0; e < m.col.size(); e++) {
+                uint32_t& slot = cnt[pos_of[m.col[e]] + 1];
+#pragma omp atomic
+                slot++;
+            }
+        }
+        for (size_t i = 0; i < H.n; i++) cnt[i + 1] += cnt[i];
+        std::unique_ptr<HostCsr> t(new HostCsr());
+        const size_t tot = cnt[H.n];
+        t->col.resize(tot); t->tag.resize(tot); t->coef.resize(tot);
+        std::vector<uint32_t> cur(cnt.begin(), cnt.end() - 1);
+        for (int w = 0; w < 3; w++) {
+            const HostCsr& m = *ms[w];
+#pragma omp parallel for schedule(static)
+            for (size_t r = 0; r < ncons; r++)
+                for (uint32_t e = m.start[r]; e < m.start[r + 1]; e++) {
+                    uint32_t at;
+                    uint32_t& slot = cur[pos_of[m.col[e]]];
+#pragma omp atomic capture
+                    at = slot++;
+                    t->col[at] = (uint32_t)r; t->tag[at] = (uint8_t)w; t->coef[at] = m.coef[e];
+                }
+        }
+        t->start = std::move(cnt);
+        out.m_t = t.release();
+        return out;
     }
     void csr_free(void* h) { delete static_cast<HostCsr*>(h); }
     Vec vspmv(const void* h, const Vec& x, size_t nout, const Fr* weights) {

@@ -94,15 +94,6 @@ struct GpuEngine {
         }
         return v;
     }
-    Vec vfrom_ptr(const Fr* h, size_t n) {
-        OpTimer ot_(c, "vfrom");
-        Vec v = alloc(n);
-        if (n) {
-            cu(cudaMemcpyAsync(v.p, h, n * sizeof(Fr), cudaMemcpyHostToDevice, c->stream), "H2D");
-            cu(cudaStreamSynchronize(c->stream), "sync");     // the caller may free h
-        }
-        return v;
-    }
     void vwrite(Vec& v, size_t at, const Fr* h, size_t n) {
         OpTimer ot_(c, "vwrite");
         if (at + n > v.n) throw MarlinError("vwrite: range out of bounds");
@@ -110,15 +101,6 @@ struct GpuEngine {
             cu(cudaMemcpyAsync(v.p + at, h, n * sizeof(Fr), cudaMemcpyHostToDevice, c->stream), "H2D");
             cu(cudaStreamSynchronize(c->stream), "sync");     // h may be a temporary
         }
-    }
-    std::vector<Fr> vhost(const Vec& v) {
-        OpTimer ot_(c, "vhost");
-        std::vector<Fr> h(v.n);
-        if (v.n) {
-            cu(cudaMemcpyAsync(h.data(), v.p, v.n * sizeof(Fr), cudaMemcpyDeviceToHost, c->stream), "D2H");
-            cu(cudaStreamSynchronize(c->stream), "sync");
-        }
-        return h;
     }
     Vec vclone(const Vec& v) {
         OpTimer ot_(c, "vclone");
@@ -250,21 +232,9 @@ struct GpuEngine {
         if (!h.empty()) cu(cudaMemcpyAsync(d, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice, c->stream), "H2D");
         return d;
     }
-    void* csr_upload(const std::vector<uint32_t>& start, const std::vector<uint32_t>& col, const std::vector<Fr>& coef,
-                     const std::vector<uint8_t>* tag) {
-        DevCsr* m = new DevCsr();
-        m->nrows = start.size() - 1;
-        m->nnz = col.size();
-        m->start = upload(start);
-        m->col = upload(col);
-        m->coef = upload(coef);
-        if (tag) m->tag = upload(*tag);
-        cu(cudaStreamSynchronize(c->stream), "sync");        // the host vectors may be temporaries
-        return m;
-    }
-    // The same, with the column and coefficient arrays written by `fill(col, coef)` straight into the context's pinned
-    // staging buffer: no zero-initialised host vectors (page faults on 40 MB per matrix at 2^20 rows) and the copy runs at
-    // the link's rate instead of the pageable path's.
+    // A CSR matrix on the device, with the column and coefficient arrays written by `fill(col, coef)` straight into the
+    // context's pinned staging buffer: no zero-initialised host vectors (page faults on 40 MB per matrix at 2^20 rows) and
+    // the copy runs at the link's rate instead of the pageable path's.
     template <class Fill>
     void* csr_upload_filled(const std::vector<uint32_t>& start, Fill&& fill) {
         const size_t nnz = start.back();
@@ -289,7 +259,6 @@ struct GpuEngine {
     }
     // Marlin's index arithmetisation on the device (index_ops.cu): joint sparsity pattern of the three uploaded matrices,
     // the six evaluation vectors on K and the column-grouped copy for the prover's t polynomial
-    static constexpr bool kDeviceIndex = true;
     struct IndexOut { size_t nnz = 0; Vec row, col, va, vb, vc, rowcol; void* m_t = nullptr; };
     IndexOut index_arith(void* ha, void* hb, void* hc, size_t ncons, size_t nvar, size_t ninst, const Domain& H) {
         OpTimer ot_(c, "index_arith");
@@ -595,11 +564,11 @@ void swb_srs_free(swb_srs* s) { srs_release(s); }
 int swb_marlin_index(swb_ctx* c, const swb_srs* srs, const swb_r1cs* cs, swb_pk** pk, swb_vk** vk) {
     if (!c || !srs || !cs || !pk || !vk) return SWB_EARG;
     if (srs->ctx != c) return swb::set_err(c, SWB_EARG, "%s", "index: the SRS was built on another context");
+    cudaSetDevice(c->device);
     std::string err;
     auto* p = new swb_pk{nullptr, nullptr};
     auto* v = new swb_vk{nullptr};
-    GpuEngine eng(c);
-    int rc = Api::index(eng, srs->h, cs->h, &p->h, &v->h, &err);
+    int rc = Api::index(srs->h, cs->h, &p->h, &v->h, &err);
     if (rc) {
         srs->h->srs->eng->msm_abandon();
         delete p;
@@ -626,9 +595,9 @@ void swb_vk_free(swb_vk* v) {
 int swb_marlin_prove(swb_ctx* c, const swb_pk* pk, const swb_r1cs* cs, swb_rng* rng, uint8_t** proof, size_t* len) {
     if (!c || !pk || !cs || !rng || !proof || !len) return SWB_EARG;
     if (pk->srs && pk->srs->ctx != c) return swb::set_err(c, SWB_EARG, "%s", "prove: the proving key belongs to another context");
+    cudaSetDevice(c->device);
     std::string err;
-    GpuEngine eng(c);
-    int rc = Api::prove(eng, pk->h, cs->h, &rng->h, proof, len, &err);
+    int rc = Api::prove(pk->h, cs->h, &rng->h, proof, len, &err);
     if (rc) {
         pk->h->pk.ck.srs->eng->msm_abandon();
         return swb::set_err(c, SWB_EINTERNAL, "prove: %s", err.c_str());
@@ -734,9 +703,10 @@ int swb_marlin_verify_proof(swb_ctx* c, const swb_vk* vk, const swb_fr* public_i
 int swb_pk_serialize(swb_ctx* c, const swb_pk* pk, const swb_vk* vk, uint8_t** bytes, size_t* len) {
     if (!c || !pk || !vk || !bytes || !len || !pk->srs) return SWB_EARG;
     if (pk->srs->ctx != c) return swb::set_err(c, SWB_EARG, "%s", "pk_serialize: the proving key belongs to another context");
+    cudaSetDevice(c->device);
     try {
-        GpuEngine eng(c);
         const UniversalSrs<GpuEngine>& srs = *pk->srs->h->srs;
+        GpuEngine& eng = *srs.eng;
         const ProvingKey<GpuEngine>& k = pk->h->pk;
         std::vector<uint8_t> out;
         const char magic[8] = {'S', 'W', 'B', 'P', 'K', '0', '0', '1'};
@@ -795,6 +765,7 @@ int swb_pk_serialize(swb_ctx* c, const swb_pk* pk, const swb_vk* vk, uint8_t** b
 
 int swb_pk_deserialize(swb_ctx* c, const uint8_t* bytes, size_t len, swb_pk** pk_out, swb_vk** vk_out) {
     if (!c || !bytes || !pk_out) return SWB_EARG;
+    cudaSetDevice(c->device);
     swb_srs* s = nullptr;
     swb_pk* p = nullptr;
     swb_vk* v = nullptr;
@@ -860,9 +831,8 @@ int swb_pk_deserialize(swb_ctx* c, const uint8_t* bytes, size_t len, swb_pk** pk
         // committer key and the index commitments together)
         p = new swb_pk{nullptr, nullptr};
         v = new swb_vk{nullptr};
-        GpuEngine eng(c);
         std::string err;
-        if (Api::index(eng, s->h, cs.get(), &p->h, &v->h, &err)) throw MarlinError("index: " + err);
+        if (Api::index(s->h, cs.get(), &p->h, &v->h, &err)) throw MarlinError("index: " + err);
         if (v->h->vk.serialize() != vkb) throw MarlinError("the key does not reproduce its verifying key");
         p->srs = s;                 // the key owns the only reference to its committer key
         *pk_out = p;

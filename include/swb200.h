@@ -146,6 +146,28 @@ int  swb_msm_g1_fr(swb_ctx*, const swb_bases*, size_t offset, const swb_fr* scal
  * callback uses the context's own communicator (swb_comm_init, below).  The callback returns 0 on success. */
 typedef int (*swb_combine_fn)(void* user, const swb_g1_jacobian* mine, swb_g1_jacobian* sum);
 int  swb_set_msm_shard(swb_ctx*, int rank, int world, swb_combine_fn combine, void* user);
+/* Multi-GPU proving from one process.  The protocol calls on ctx (swb_marlin_index, swb_marlin_prove,
+ * swb_pk_deserialize) share each commit / open MSM between ctx (rank 0) and the n_peers other contexts (ranks
+ * 1..n_peers), in this process, on any devices, the same device included.  The split is swb_set_msm_shard's for a
+ * world of 1 + n_peers: by bucket in a power-of-two world once the SRS powers have window tables, by index range
+ * otherwise.  For every MSM the scalars a peer reads (all of them by bucket, its slice by index) are copied to its
+ * device with cudaMemcpyPeerAsync (direct where the devices allow peer access, which this call enables for the
+ * process, staged through the host elsewhere), the share runs on the peer's own stream and MSM slots, and ctx adds the
+ * shares on the host.  The calling thread launches on every device and only waits for the results; the NTTs and
+ * polynomial work stay on ctx.  Proof and key bytes are those of one GPU.  n_peers = 0 detaches.  Refused (SWB_EARG)
+ * while ctx shards through swb_set_msm_shard or is itself a peer, for a peer that has peers or a shard of its own, for
+ * ctx itself or a repeated peer, and while an MSM is in flight; swb_set_msm_shard in turn refuses ctx and its peers.
+ * The peers plan their shares with ctx's MSM settings (swb_msm_set_window_bits, _set_table_policy, _set_pair_sums),
+ * whatever their own are, so that all ranks decompose the scalars alike.
+ * Lifetimes: the first sharded MSM over an SRS's powers copies them to every peer (replicas, which later receive the
+ * SRS's window tables by copy too; a peer without room for the tables keeps that SRS's MSMs on index-range shares); the
+ * SRS owns its replicas and frees them on the peer contexts when it is freed.  So the peers must outlive every SRS and
+ * proving key created on ctx.  Contexts may then be destroyed in any order: swb_destroy of ctx or of a peer detaches
+ * it from the other side.  A peer is busy while ctx's call runs: no other thread may use it then.  Not shared:
+ * swb_marlin_verify_batch, the swb_msm_g1* calls, NTTs and polynomial work. */
+int  swb_set_msm_peers(swb_ctx*, swb_ctx* const* peers, int n_peers);
+/* bytes ctx has copied to its peers since it was created: SRS replicas and MSM scalars */
+uint64_t swb_peer_copy_bytes(const swb_ctx*);
 /* ---- multi-GPU exchange inside the library (one process per GPU; NCCL resolved at run time) ---------------
  * swb_comm_unique_id: rank 0 obtains the 128-byte ncclUniqueId and hands it to the other ranks out of band
  * (any channel: a file, MPI, torch.distributed's store); swb_comm_init: every rank joins, on its context's

@@ -24,7 +24,7 @@ SYMBOLS = [
     "swb_profile_enable", "swb_profile_last",
     "swb_bases_load", "swb_bases_load_dev", "swb_bases_from_powers", "swb_bases_export", "swb_bases_precompute", "swb_bases_table_info",
     "swb_bases_len", "swb_bases_free",
-    "swb_msm_g1", "swb_msm_g1_dev", "swb_msm_g1_fr_dev", "swb_msm_g1_fr", "swb_msm_g1_batch_dev", "swb_set_msm_shard", "swb_comm_unique_id", "swb_comm_init", "swb_comm_info", "swb_comm_sum_g1", "swb_comm_destroy", "swb_msm_plan", "swb_msm_set_window_bits", "swb_msm_set_table_policy", "swb_msm_set_pair_sums", "swb_msm_set_bucket_shard", "swb_g1_sum_jacobian",
+    "swb_msm_g1", "swb_msm_g1_dev", "swb_msm_g1_fr_dev", "swb_msm_g1_fr", "swb_msm_g1_batch_dev", "swb_set_msm_shard", "swb_set_msm_peers", "swb_peer_copy_bytes", "swb_comm_unique_id", "swb_comm_init", "swb_comm_info", "swb_comm_sum_g1", "swb_comm_destroy", "swb_msm_plan", "swb_msm_set_window_bits", "swb_msm_set_table_policy", "swb_msm_set_pair_sums", "swb_msm_set_bucket_shard", "swb_g1_sum_jacobian",
     "swb_fixed_base_powers",
     "swb_ntt_fr", "swb_ntt_fr_dev", "swb_ntt_fr_batch_dev",
     "swb_rng_test_rng", "swb_rng_from_seed", "swb_rng_from_entropy", "swb_rng_next_u64", "swb_rng_free",
@@ -86,6 +86,8 @@ def load() -> ctypes.CDLL:
         "swb_bases_free": (None, [vp]),
         "swb_msm_g1_batch_dev": (i32, [vp, vp, vp, vp, vp, sz, i32, vp]),
         "swb_set_msm_shard": (i32, [vp, i32, i32, vp, vp]),
+        "swb_set_msm_peers": (i32, [vp, pvp, i32]),
+        "swb_peer_copy_bytes": (ctypes.c_uint64, [vp]),
         "swb_comm_unique_id": (i32, [ctypes.c_char_p]),
         "swb_comm_init": (i32, [vp, ctypes.c_char_p, i32, i32]),
         "swb_comm_info": (i32, [vp, ctypes.POINTER(i32), ctypes.POINTER(i32)]),

@@ -299,6 +299,19 @@ class Backend:
         self._combine_cb = cb_t(combine)        # keep the trampoline alive
         self._check(self._lib.swb_set_msm_shard(self._h, rank, world, ctypes.cast(self._combine_cb, ctypes.c_void_p), None))
 
+    def set_msm_peers(self, peers):
+        """Multi-GPU proving from one process (swb_set_msm_peers): every commit / open MSM of the Marlin entry points on
+        this backend is shared with the backends in `peers` (other devices, or the same one), which take ranks
+        1..len(peers).  The peers are kept alive as long as this backend; an empty list detaches."""
+        peers = list(peers)
+        arr = (ctypes.c_void_p * max(len(peers), 1))(*[p._h.value for p in peers])
+        self._check(self._lib.swb_set_msm_peers(self._h, arr, len(peers)))
+        self._peers = peers                     # the SRS replicas on the peers are freed with this backend's handles
+
+    def peer_copy_bytes(self) -> int:
+        """bytes this backend has copied to its peers (SRS replicas and MSM scalars)"""
+        return int(self._lib.swb_peer_copy_bytes(self._h))
+
     def set_msm_window_bits(self, c: int):
         self._check(self._lib.swb_msm_set_window_bits(self._h, c))
 

@@ -1,4 +1,5 @@
 // Context, error reporting, device buffers.
+#include <algorithm>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstring>
@@ -170,6 +171,10 @@ void swb_destroy(swb_ctx* c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     swb_comm_destroy(c);
+    // unlink from the peer relation on both sides, whichever context goes first
+    for (swb_ctx* p : c->msm_peers) p->msm_primaries.erase(std::find(p->msm_primaries.begin(), p->msm_primaries.end(), c));
+    for (swb_ctx* q : c->msm_primaries) q->msm_peers.erase(std::find(q->msm_peers.begin(), q->msm_peers.end(), c));
+    if (c->peer_ev) cudaEventDestroy(c->peer_ev);
     for (auto& kv : c->vec_cache) cudaFree(kv.second);
     for (auto& sl : c->msm_slot) {
         if (sl.work) { cudaStreamSynchronize(sl.work); cudaStreamDestroy(sl.work); }

@@ -69,6 +69,7 @@ struct swb_ctx {
     struct MsmRequest {
         const swb_bases* bases; size_t offset, n; const void* scalars; int montgomery; swb::BucketShard shard;
         int slot = -1;                 // -1: noted; else the slot it was launched on
+        bool single = false;           // noted, and its run could not go out as one batch: launched on its own
         bool done = false;             // finished: the result is in `out`
         swb_g1_jacobian out;
     };
@@ -81,6 +82,12 @@ struct swb_ctx {
     int shard_rank = 0, shard_world = 1;
     int (*shard_combine)(void*, const swb_g1_jacobian*, swb_g1_jacobian*) = nullptr;
     void* shard_user = nullptr;
+    // swb_set_msm_peers: contexts of this process that take ranks 1..n of every prover MSM (this context is rank 0),
+    // and the contexts that have this one as a peer (swb_destroy of either side unlinks it)
+    std::vector<swb_ctx*> msm_peers;
+    std::vector<swb_ctx*> msm_primaries;
+    cudaEvent_t peer_ev = nullptr;     // orders a copy to a peer after the work queued on `stream`
+    uint64_t peer_bytes = 0;           // bytes copied to the peers (swb_peer_copy_bytes)
 
     // swb_comm_*: NCCL communicator of this context (one process per GPU), staging buffers of the all-gather
     void* comm = nullptr;
@@ -117,6 +124,10 @@ void sync_all_streams(swb_ctx* c);
 int msm_queue_submit(swb_ctx* c, const swb_bases* bases, size_t offset, const void* scalars_dev, size_t n, int montgomery,
                      BucketShard shard, size_t* id);
 int msm_queue_flush(swb_ctx* c);
+// launches the next run of noted requests: a batch, or one request on the next slot of 1 and 2 once that slot's previous
+// MSM has finished.  *launched = false when nothing is noted.  A flush launches until nothing is; a caller that drives
+// several contexts launches a run on each in turn, so that their devices work at once.
+int msm_queue_launch(swb_ctx* c, bool* launched);
 // flushes when the request is still noted, waits for it and hands its result over (once)
 int msm_queue_result(swb_ctx* c, size_t id, swb_g1_jacobian* out);
 // launches and finishes every request, keeping the results (before the bases they read are replaced)

@@ -2,6 +2,8 @@
 // CUDA engine.  Host orchestration (transcript, AHP rounds, KZG bookkeeping) is marlin/marlin.hpp;
 // every NTT, MSM and fixed-base table goes to the kernels of this library -- there is no CPU
 // engine in libswb200.
+#include <set>
+
 #include "ctx.hpp"
 #include "marlin/c_api_impl.hpp"
 #include "index_ops.hpp"
@@ -362,7 +364,17 @@ struct GpuEngine {
             memcpy(out[i].y.l, tmp[i].y.l, 48);
         }
     }
-    void free_bases(void* h) { swb_bases_free(static_cast<swb_bases*>(h)); }
+    // the bases and their replicas on the peers
+    void free_bases(void* h) {
+        for (auto it = replicas.begin(); it != replicas.end();) {
+            if (it->first.first != h) { ++it; continue; }
+            OnDevice d(it->first.second->device);
+            swb_bases_free(it->second);
+            it = replicas.erase(it);
+        }
+        no_peer_tables.erase(static_cast<const swb_bases*>(h));
+        swb_bases_free(static_cast<swb_bases*>(h));
+    }
     // window tables (swb_bases_precompute) with the digit width that suits MSMs of about typical_n
     // scalars (tables_pick_window).  KZG powers lie in the prime-order subgroup (g is cofactor-cleared), which the
     // tables require.
@@ -381,65 +393,223 @@ struct GpuEngine {
         if (swb_bases_precompute(c, b, best) != SWB_OK) {                     // keep going on the plain path
             cudaGetLastError();
             if (c->trace) fprintf(stderr, "[swb trace] SRS window tables not built: %s\n", swb_last_error(c));
+            return;
         }
+        peer_tables(b);                                                        // the peers get the levels by copy
     }
     // The MSMs of a round (the commitments, the parts of an opening) go to the context's MSM queue (ctx.hpp:
     // msm_queue_*), which batches them over window tables or overlaps them on its slots.  What the engine adds is the
     // sharding over ranks: each rank submits its share of every MSM, and the shares are summed when a result is asked
-    // for.  The scalars must stay alive until the result has been taken.
+    // for.  The ranks are either processes (swb_set_msm_shard: every process runs the prover, this context is one
+    // rank) or the peer contexts of this one (swb_set_msm_peers: this context is rank 0 and submits every other
+    // rank's share to that rank's queue, with a copy of the scalars on the rank's device).  The scalars must stay
+    // alive until the result has been taken.
+    struct PeerShare {
+        swb_ctx* ctx;
+        size_t id = 0;                     // in the peer's queue
+        void* buf = nullptr;               // the peer's copy of the scalars (a block of its vector cache)
+        size_t blk = 0;
+    };
     struct Ticket {
         bool sharded, combined;
         G1Point value;                     // the sum over the ranks, once combined
+        std::vector<PeerShare> peers;      // ranks 1.. when they are peer contexts
     };
     std::map<size_t, Ticket> tickets;      // by queue id; erased when msm_result hands the value over
-    bool sharding() const { return c->shard_world > 1 && (c->shard_combine || c->comm); }
+    // copies of the SRS powers (and later of their window tables) on each peer, by (bases, peer); freed with the bases
+    std::map<std::pair<const swb_bases*, swb_ctx*>, swb_bases*> replicas;
+    // bases whose window tables could not be copied to every peer: their MSMs are shared by index range
+    std::set<const swb_bases*> no_peer_tables;
+    // the ranks every MSM is shared over, and this context's rank
+    int world() const { return c->msm_peers.empty() ? c->shard_world : 1 + (int)c->msm_peers.size(); }
+    int rank() const { return c->msm_peers.empty() ? c->shard_rank : 0; }
+    bool sharding() const { return world() > 1 && (!c->msm_peers.empty() || c->shard_combine || c->comm); }
     // Power-of-two worlds shard by BUCKET (swb::BucketShard: every rank sees the whole polynomial -- it
     // has it anyway -- and fills its interleaved share of the buckets, so accumulation AND bucket reduction shrink
     // and the window width stays that of one GPU); other worlds by contiguous index range.
-    bool shards_by_bucket() const { return sharding() && (c->shard_world & (c->shard_world - 1)) == 0; }
+    bool shards_by_bucket() const { return sharding() && (world() & (world() - 1)) == 0; }
     // (only over bases with window tables: on the plain path every rank would still sort all pairs, and the index
     // split measured slightly faster -- 2^20 constraints on two GPUs: 0.248 s against 0.256 s)
-    bool bucket_mode(const swb_bases* b) const { return shards_by_bucket() && b && b->tab_w > 0; }
-    // the bucket shard an MSM runs under: this rank's share when it shards by bucket, else the context's own
-    BucketShard bucket_shard(bool by_bucket) const {
-        return by_bucket ? BucketShard{c->shard_rank, c->shard_world} : BucketShard{c->bucket_rank, c->bucket_world};
+    bool bucket_mode(const swb_bases* b) const { return shards_by_bucket() && b && b->tab_w > 0 && !no_peer_tables.count(b); }
+    // the bucket shard an MSM of rank r runs under: r's share when it shards by bucket, else the context's own
+    BucketShard bucket_shard(bool by_bucket, int r) const {
+        return by_bucket ? BucketShard{r, world()} : BucketShard{c->bucket_rank, c->bucket_world};
     }
-    // this rank's part [lo, lo + count) of an MSM of n scalars sharded by index (remainder to the first ranks): the count
-    size_t local_part(size_t n, size_t* lo) const {
-        const size_t base = n / (size_t)c->shard_world, rem = n % (size_t)c->shard_world, r = (size_t)c->shard_rank;
-        *lo = r * base + (r < rem ? r : rem);
-        return base + (r < rem ? 1 : 0);
+    // rank r's part [lo, lo + count) of an MSM of n scalars sharded by index (remainder to the first ranks): the count
+    size_t local_part(size_t n, int r, size_t* lo) const {
+        const size_t w = (size_t)world(), base = n / w, rem = n % w, rr = (size_t)r;
+        *lo = rr * base + (rr < rem ? rr : rem);
+        return base + (rr < rem ? 1 : 0);
+    }
+    // the peer calls below run on the peer's device; the engine's own work expects this context's
+    struct OnDevice {
+        int prev = 0;
+        explicit OnDevice(int d) { cudaGetDevice(&prev); cudaSetDevice(d); }
+        ~OnDevice() { cudaSetDevice(prev); }
+    };
+    // ... and plans its shares with this context's MSM settings (window width, table policy, pair sums): by bucket the
+    // shares add up to the MSM only when every rank takes the same digit width and the same path, and with the same
+    // requests in its queue a peer then also batches as this context does.  The peer's own settings come back after.
+    struct AsPeer : OnDevice {
+        swb_ctx* p;
+        int win, tab, pair;
+        AsPeer(swb_ctx* peer, const swb_ctx* c)
+            : OnDevice(peer->device), p(peer), win(peer->msm_window_override), tab(peer->msm_table_policy), pair(peer->msm_pair_policy) {
+            p->msm_window_override = c->msm_window_override;
+            p->msm_table_policy = c->msm_table_policy;
+            p->msm_pair_policy = c->msm_pair_policy;
+        }
+        ~AsPeer() {
+            p->msm_window_override = win;
+            p->msm_table_policy = tab;
+            p->msm_pair_policy = pair;
+        }
+    };
+    void ck_peer(swb_ctx* p, int rc, const char* what) {
+        if (rc != SWB_OK) throw MarlinError(std::string(what) + " (peer context on device " + std::to_string(p->device) + "): " + swb_last_error(p));
+    }
+    // b's replica on peer p, created by a device-to-device copy of the records: level 0 (what index-range shares read),
+    // or with `tables` the window-table levels too (bucket shares), which need half of the peer's free memory as
+    // bases_tune asks on this device.  The copy runs on this context's stream, which produced b, and has finished when
+    // this returns.
+    swb_bases* replica(const swb_bases* b, swb_ctx* p, bool tables) {
+        swb_bases*& r = replicas[{b, p}];
+        const int tab_w = tables ? b->tab_w : 0;
+        if (r && r->n == b->n && (tab_w == 0 || (r->tab_c == b->tab_c && r->tab_w == b->tab_w))) return r;
+        const size_t bytes = b->n * (size_t)(tab_w > 0 ? tab_w : 1) * 96;
+        swb::Fq* xy = nullptr;
+        {
+            OnDevice d(p->device);
+            size_t free_b = 0, total_b = 0;
+            if ((tab_w > 0 && (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || bytes > free_b / 2)) ||
+                cudaMalloc(&xy, bytes ? bytes : 96) != cudaSuccess) {
+                cudaGetLastError();
+                throw MarlinError("msm: no room for the SRS powers (" + std::to_string(bytes) + " B) on the peer context on device " +
+                                  std::to_string(p->device));
+            }
+        }
+        cudaError_t e = bytes ? cudaMemcpyPeerAsync(xy, p->device, b->xy, c->device, bytes, c->stream) : cudaSuccess;
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        if (e != cudaSuccess) {
+            OnDevice d(p->device);
+            cudaFree(xy);
+            cu(e, "msm: copying the SRS powers to a peer");
+        }
+        c->peer_bytes += bytes;
+        if (!r) {
+            r = new swb_bases();
+            r->ctx = p;
+        } else {
+            OnDevice d(p->device);
+            sync_all_streams(p);             // the peer's MSMs over the old records have finished
+            cudaFree(r->xy);
+        }
+        r->xy = xy;
+        r->n = b->n;
+        r->tab_c = tab_w > 0 ? b->tab_c : 0;
+        r->tab_w = tab_w;
+        return r;
+    }
+    // Bucket shares need b's window tables on every peer: copied here.  A peer without room for them sends b's MSMs back
+    // to index-range shares (every replica holds level 0) instead of failing every later call.
+    bool peer_tables(const swb_bases* b) {
+        if (no_peer_tables.count(b)) return false;
+        for (swb_ctx* p : c->msm_peers) {
+            try {
+                replica(b, p, true);
+            } catch (const MarlinError& e) {
+                if (c->trace) fprintf(stderr, "[swb trace] SRS window tables not copied to a peer, sharing by index range: %s\n", e.what());
+                no_peer_tables.insert(b);
+                return false;
+            }
+        }
+        return true;
+    }
+    // rank r's share of an MSM of n scalars on its peer context: the scalars it reads go to a block of the peer's vector
+    // cache (all of them by bucket, its slice by index), copied after the work queued so far on this context's stream.
+    // The share joins the ticket first, so that msm_abandon hands the block back whatever fails here.
+    void peer_submit(Ticket& t, int r, const swb_bases* b, size_t offset, const Vec& scalars, size_t n, bool by_bucket) {
+        swb_ctx* p = c->msm_peers[r - 1];
+        swb_bases* rb = replica(b, p, by_bucket);
+        size_t lo = 0;
+        if (!by_bucket) n = local_part(n, r, &lo);
+        t.peers.push_back(PeerShare{p});
+        PeerShare& s = t.peers.back();
+        if (n) cu(cudaEventRecord(c->peer_ev, c->stream), "msm: event");
+        OnDevice d(p->device);
+        if (n) {
+            s.buf = vec_alloc(p, n * sizeof(Fr), &s.blk);
+            if (!s.buf) ck_peer(p, SWB_ENOMEM, "msm");
+            cu(cudaStreamWaitEvent(p->stream, c->peer_ev, 0), "msm: event");
+            cu(cudaMemcpyPeerAsync(s.buf, p->device, scalars.p + lo, c->device, n * sizeof(Fr), p->stream), "msm: copying scalars to a peer");
+            c->peer_bytes += n * sizeof(Fr);
+        }
+        ck_peer(p, msm_queue_submit(p, rb, offset + lo, s.buf, n, 1, bucket_shard(by_bucket, r), &s.id), "msm");
+    }
+    // hands the peer's copy of the scalars back to its vector cache (its MSM has finished or was abandoned)
+    static void release(PeerShare& s) {
+        if (!s.buf) return;
+        OnDevice d(s.ctx->device);           // vec_free may hand the cache back to the peer's device
+        vec_free(s.ctx, s.buf, s.blk);
+        s.buf = nullptr;
     }
     // shares -> sums over all ranks.  With the library's communicator every share that is outstanding (the
     // commitments of a round are all submitted before the first result is asked for) goes into ONE all-gather;
-    // a caller-supplied callback is invoked per MSM.
+    // a caller-supplied callback is invoked per MSM.  With peer contexts every queue is launched first, a run per
+    // context in turn, so that all devices work at once; then the shares are taken and added on the host.
     void combine_pending() {
         std::vector<size_t> ids;
         for (auto& kv : tickets)
             if (kv.second.sharded && !kv.second.combined) ids.push_back(kv.first);
         std::vector<swb_g1_jacobian> mine(ids.size()), sums(ids.size());
+        if (!c->msm_peers.empty()) {
+            for (bool more = true; more;) {
+                more = false;
+                for (swb_ctx* p : c->msm_peers) {
+                    AsPeer as(p, c);
+                    bool launched = false;
+                    ck_peer(p, msm_queue_launch(p, &launched), "msm");
+                    more |= launched;
+                }
+                bool launched = false;
+                ck(msm_queue_launch(c, &launched), "msm");
+                more |= launched;
+            }
+        }
         for (size_t k = 0; k < ids.size(); k++) ck(msm_queue_result(c, ids[k], &mine[k]), "msm");
-        if (c->shard_combine) {
+        if (!c->msm_peers.empty()) {
+            for (size_t k = 0; k < ids.size(); k++) {
+                std::vector<swb_g1_jacobian> parts(1, mine[k]);
+                for (PeerShare& s : tickets.at(ids[k]).peers) {
+                    AsPeer as(s.ctx, c);
+                    parts.emplace_back();
+                    ck_peer(s.ctx, msm_queue_result(s.ctx, s.id, &parts.back()), "msm");
+                    release(s);
+                }
+                ck(swb_g1_sum_jacobian(c, parts.data(), parts.size(), &sums[k]), "msm (sum of the peers' shares)");
+            }
+        } else if (c->shard_combine) {
             for (size_t k = 0; k < ids.size(); k++)
                 if (c->shard_combine(c->shard_user, &mine[k], &sums[k]) != 0) throw MarlinError("msm: combining the ranks' partial results failed");
         } else {
             ck(comm_sum_g1(c, mine.data(), mine.size(), sums.data()), "msm (all-gather of the partial results)");
         }
-        for (size_t k = 0; k < ids.size(); k++) tickets.at(ids[k]) = Ticket{true, true, from_jacobian(sums[k])};
+        for (size_t k = 0; k < ids.size(); k++) tickets.at(ids[k]) = Ticket{true, true, from_jacobian(sums[k]), {}};
     }
     // (sizes the SRS window tables: in a power-of-two world they will be used by bucket, i.e. on whole polynomials)
     size_t msm_local_count(size_t n) {
         size_t lo;
-        return !sharding() || shards_by_bucket() ? n : local_part(n, &lo);
+        return !sharding() || shards_by_bucket() ? n : local_part(n, rank(), &lo);
     }
     size_t msm_submit(void* h, size_t offset, const Vec& scalars, size_t n) {
         OpTimer ot_(c, "msm_submit");
         const swb_bases* b = static_cast<swb_bases*>(h);
-        const bool sharded = sharding(), by_bucket = bucket_mode(b);
-        size_t lo = 0, id = 0;
-        if (sharded && !by_bucket) n = local_part(n, &lo);
-        ck(msm_queue_submit(c, b, offset + lo, scalars.p + lo, n, 1, bucket_shard(by_bucket), &id), "msm");
-        tickets[id] = Ticket{sharded, false, G1Point::identity()};
+        const bool sharded = sharding(), by_bucket = bucket_mode(b) && peer_tables(b);
+        size_t lo = 0, id = 0, mine = n;
+        if (sharded && !by_bucket) mine = local_part(n, rank(), &lo);
+        ck(msm_queue_submit(c, b, offset + lo, scalars.p + lo, mine, 1, bucket_shard(by_bucket, rank()), &id), "msm");
+        Ticket& t = tickets[id] = Ticket{sharded, false, G1Point::identity(), {}};
+        for (int r = 1; sharded && r <= (int)c->msm_peers.size(); r++) peer_submit(t, r, b, offset, scalars, n, by_bucket);
         return id;
     }
     G1Point msm_result(size_t id) {
@@ -456,10 +626,26 @@ struct GpuEngine {
         tickets.erase(id);
         return v;
     }
-    // the tables replace the bases: every MSM must have finished (the results stay in the queue)
-    void msm_drain() { ck(msm_queue_drain(c), "msm"); }
+    // the tables replace the bases: every MSM must have finished, on the peers too (the results stay in the queues)
+    void msm_drain() {
+        for (swb_ctx* p : c->msm_peers) {
+            AsPeer as(p, c);
+            ck_peer(p, msm_queue_drain(p), "msm");
+        }
+        ck(msm_queue_drain(c), "msm");
+    }
     // after a failed call: the MSMs of the call are forgotten, their scalars are gone
-    void msm_abandon() { tickets.clear(); msm_queue_abandon(c); }
+    void msm_abandon() {
+        for (swb_ctx* p : c->msm_peers) {
+            OnDevice d(p->device);
+            msm_queue_abandon(p);
+            sync_all_streams(p);             // copies whose MSM never launched may still be reading our scalars
+        }
+        for (auto& kv : tickets)
+            for (PeerShare& s : kv.second.peers) release(s);
+        tickets.clear();
+        msm_queue_abandon(c);
+    }
 };
 using Api = MarlinApi<GpuEngine>;
 

@@ -28,6 +28,7 @@
 //
 // The result is the affine value (as a Z = 1 Jacobian), which is unique, hence bit-identical to
 // what arkworks' callers see after into_affine().
+#include <algorithm>
 #include <memory>
 
 #include "msm_common.cuh"
@@ -310,23 +311,30 @@ int msm_queue_submit(swb_ctx* c, const swb_bases* bases, size_t offset, const vo
     return SWB_OK;
 }
 
-// finishes the request running on slot s, if there is one
+// finishes the MSM running on slot s, if there is one, and hands its results to the requests it serves (a batch on slot
+// 0 serves several, in submission order)
 static int msm_queue_collect(swb_ctx* c, int s) {
+    if (!c->msm_slot[s].active) return SWB_OK;
+    swb_g1_jacobian outs[MSM_MAX_BATCH];
+    const int rc = msm_end(c, s, outs);
+    int k = 0;
     for (auto& kv : c->msm_queue) {
         swb_ctx::MsmRequest& r = kv.second;
         if (r.slot != s || r.done) continue;
-        const int rc = msm_end(c, s, &r.out);
+        r.out = outs[k++];
         r.done = rc == SWB_OK;
-        return rc;
     }
-    return SWB_OK;
+    return rc;
 }
 
-int msm_queue_flush(swb_ctx* c) {
+int msm_queue_launch(swb_ctx* c, bool* launched) {
+    *launched = false;
     auto it = c->msm_queue.begin();
-    while (it != c->msm_queue.end()) {
-        const swb_ctx::MsmRequest& first = it->second;
-        if (first.slot >= 0) { ++it; continue; }
+    while (it != c->msm_queue.end() && it->second.slot >= 0) ++it;
+    if (it == c->msm_queue.end()) return SWB_OK;
+    *launched = true;
+    swb_ctx::MsmRequest& first = it->second;
+    if (!first.single) {
         swb_ctx::MsmRequest* run[MSM_MAX_BATCH];
         size_t offs[MSM_MAX_BATCH], ns[MSM_MAX_BATCH];
         const void* scs[MSM_MAX_BATCH];
@@ -339,25 +347,31 @@ int msm_queue_flush(swb_ctx* c) {
             run[cnt] = &r;
             offs[cnt] = r.offset; ns[cnt] = r.n; scs[cnt] = r.scalars;
         }
-        int rc = SWB_OK;
         if (cnt >= 2 && msm_can_batch(c, first.bases, cnt, ns)) {
-            // the batch runs on the context's stream with slot 0's scratch: the other slots finish first
-            for (int s = 1; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
-            swb_g1_jacobian outs[MSM_MAX_BATCH];
+            // the batch runs on the context's stream with slot 0's scratch: the other slots and the previous batch finish
+            // first.  Its results are collected when one of them is asked for.
+            int rc = SWB_OK;
+            for (int s = 0; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
             if (rc == SWB_OK) rc = msm_begin_batch(c, 0, first.bases, cnt, offs, scs, ns, first.montgomery, first.shard);
-            if (rc == SWB_OK) rc = msm_end(c, 0, outs);
             if (rc != SWB_OK) return rc;
-            for (size_t k = 0; k < cnt; k++) { run[k]->slot = 0; run[k]->done = true; run[k]->out = outs[k]; }
-            continue;
+            for (size_t k = 0; k < cnt; k++) run[k]->slot = 0;
+            return SWB_OK;
         }
-        for (size_t k = 0; k < cnt; k++) {
-            const int s = c->msm_next_slot;
-            c->msm_next_slot = s == 1 ? 2 : 1;
-            rc = msm_queue_collect(c, s);
-            if (rc == SWB_OK) rc = msm_begin(c, s, run[k]->bases, run[k]->offset, run[k]->scalars, run[k]->n, run[k]->montgomery, run[k]->shard);
-            if (rc != SWB_OK) return rc;
-            run[k]->slot = s;
-        }
+        for (size_t k = 0; k < cnt; k++) run[k]->single = true;      // this run goes out one request at a time
+    }
+    const int s = c->msm_next_slot;
+    c->msm_next_slot = s == 1 ? 2 : 1;
+    int rc = msm_queue_collect(c, s);
+    if (rc == SWB_OK) rc = msm_begin(c, s, first.bases, first.offset, first.scalars, first.n, first.montgomery, first.shard);
+    if (rc != SWB_OK) return rc;
+    first.slot = s;
+    return SWB_OK;
+}
+
+int msm_queue_flush(swb_ctx* c) {
+    for (bool launched = true; launched;) {
+        const int rc = msm_queue_launch(c, &launched);
+        if (rc != SWB_OK) return rc;
     }
     return SWB_OK;
 }
@@ -375,15 +389,15 @@ int msm_queue_result(swb_ctx* c, size_t id, swb_g1_jacobian* out) {
 
 int msm_queue_drain(swb_ctx* c) {
     int rc = msm_queue_flush(c);
-    for (int s = 1; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
+    for (int s = 0; s < swb_ctx::MSM_SLOTS && rc == SWB_OK; s++) rc = msm_queue_collect(c, s);
     return rc;
 }
 
 void msm_queue_abandon(swb_ctx* c) {
     const std::string err = c->err;         // the failure that led here stays the context's last error
-    swb_g1_jacobian dummy;
+    swb_g1_jacobian dummy[MSM_MAX_BATCH];                       // slot 0 may hold a batch
     for (int s = 0; s < swb_ctx::MSM_SLOTS; s++)
-        if (c->msm_slot[s].active) msm_end(c, s, &dummy);       // waits for the slot's work
+        if (c->msm_slot[s].active) msm_end(c, s, dummy);        // waits for the slot's work
     c->msm_queue.clear();
     c->err = err;
 }
@@ -550,12 +564,57 @@ int swb_set_msm_shard(swb_ctx* c, int rank, int world, swb_combine_fn combine, v
         return SWB_OK;
     }
     SWB_REQUIRE(c, rank >= 0 && rank < world, "set_msm_shard: rank out of range");
+    SWB_REQUIRE(c, c->msm_peers.empty() && c->msm_primaries.empty(), "set_msm_shard: the context shares its MSMs with peer contexts (swb_set_msm_peers)");
     // without a callback the partial results travel through the context's own communicator (swb_comm_init)
     SWB_REQUIRE(c, combine || (c->comm && c->comm_world == world && c->comm_rank == rank),
                 "set_msm_shard: no combine callback and no communicator of this shape (swb_comm_init)");
     c->shard_rank = rank; c->shard_world = world; c->shard_combine = combine; c->shard_user = user;
     return SWB_OK;
 }
+
+int swb_set_msm_peers(swb_ctx* c, swb_ctx* const* peers, int n_peers) {
+    if (!c) return SWB_EARG;
+    SWB_REQUIRE(c, n_peers >= 0 && n_peers < 1024 && (n_peers == 0 || peers), "set_msm_peers: bad peer list");
+    auto idle = [](const swb_ctx* x) {
+        for (auto& sl : x->msm_slot)
+            if (sl.active) return false;
+        return x->msm_queue.empty();
+    };
+    SWB_REQUIRE(c, idle(c), "set_msm_peers: an MSM is in flight");
+    for (swb_ctx* p : c->msm_peers) SWB_REQUIRE(c, idle(p), "set_msm_peers: an MSM is in flight on a peer");
+    if (n_peers > 0) {
+        SWB_REQUIRE(c, c->shard_world <= 1, "set_msm_peers: the context shards through swb_set_msm_shard");
+        SWB_REQUIRE(c, c->msm_primaries.empty(), "set_msm_peers: the context is a peer of another context");
+    }
+    for (int i = 0; i < n_peers; i++) {
+        const swb_ctx* p = peers[i];
+        SWB_REQUIRE(c, p != nullptr, "set_msm_peers: NULL peer");
+        SWB_REQUIRE(c, p != c, "set_msm_peers: a context cannot be its own peer");
+        for (int j = 0; j < i; j++) SWB_REQUIRE(c, peers[j] != p, "set_msm_peers: repeated peer");
+        SWB_REQUIRE(c, p->msm_peers.empty() && p->shard_world <= 1, "set_msm_peers: a peer has peers or a shard of its own");
+        SWB_REQUIRE(c, idle(p), "set_msm_peers: an MSM is in flight on a peer");
+    }
+    if (n_peers > 0 && !c->peer_ev) {
+        SWB_CUDA(c, cudaSetDevice(c->device));
+        SWB_CUDA(c, cudaEventCreateWithFlags(&c->peer_ev, cudaEventDisableTiming));
+    }
+    // direct access between the devices where they allow it; elsewhere cudaMemcpyPeerAsync stages through the host
+    for (int i = 0; i < n_peers; i++) {
+        const int a = c->device, b = peers[i]->device;
+        int ab = 0, ba = 0;
+        if (a == b || cudaDeviceCanAccessPeer(&ab, a, b) != cudaSuccess || cudaDeviceCanAccessPeer(&ba, b, a) != cudaSuccess) continue;
+        if (ab && cudaSetDevice(a) == cudaSuccess) cudaDeviceEnablePeerAccess(b, 0);
+        if (ba && cudaSetDevice(b) == cudaSuccess) cudaDeviceEnablePeerAccess(a, 0);
+        cudaGetLastError();              // cudaErrorPeerAccessAlreadyEnabled, or access refused: the copies are staged
+    }
+    cudaSetDevice(c->device);
+    for (swb_ctx* p : c->msm_peers) p->msm_primaries.erase(std::find(p->msm_primaries.begin(), p->msm_primaries.end(), c));
+    c->msm_peers.assign(peers, peers + n_peers);
+    for (swb_ctx* p : c->msm_peers) p->msm_primaries.push_back(c);
+    return SWB_OK;
+}
+
+uint64_t swb_peer_copy_bytes(const swb_ctx* c) { return c ? c->peer_bytes : 0; }
 
 int swb_msm_set_bucket_shard(swb_ctx* c, int rank, int world) {
     if (!c) return SWB_EARG;
